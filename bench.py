@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # our arm (CUDA, through the C ABI)
   python bench.py --impl reference --gpus N --steps K ...  # CPU arm: the oracle port on all host cores
+  python bench.py ... --dump-outputs DIR                   # also save what the last timed step computed (dump_outputs)
   (N > 1: launched by torch.distributed.run, one rank per GPU)
 
 Workload (BASELINE.json configs[1]): T04_2D_reg_test_large_grid / bench06 homogeneous box
@@ -252,6 +253,31 @@ def emit(line):
     out = _REAL_STDOUT or sys.stdout
     out.write(json.dumps(line) + "\n")
     out.flush()
+
+
+# At most this many nodes are dumped over all ranks: State (3 f64), particle u[5] (5 f64), the particle's clock t,
+# step size dt, flags and status (f64 each) and the node index come to 104 B a node, 55 MB here, under the 64 MB the
+# dump may take.
+DUMP_NODES = 1 << 19
+
+
+def dump_outputs(out_dir, eng, counters, max_nodes=DUMP_NODES, suffix=""):
+    """--dump-outputs: what the timed path computed in its last step, as float64 .npy files in out_dir, so that two
+    builds run with the same arguments (hence the same inputs) can be compared output for output.  State (3, n), the
+    particles' u[5] (5, n), t, dt, flags and status (n each) at n nodes: every node of the strip when it has at most
+    max_nodes, else a sample of max_nodes drawn with a fixed seed, its flat (row-major) indices in node_index (n).
+    counters: the step's integer counters in picles_counters_t order, timings left out."""
+    S = eng.state().reshape(3, -1)
+    p = eng.particles()
+    n = S.shape[1]
+    idx = np.arange(n) if n <= max_nodes else np.sort(np.random.default_rng(0).choice(n, max_nodes, replace=False))
+    arrays = {"state": S[:, idx], "particles_u": p["z"].reshape(5, -1)[:, idx],
+              **{"particles_" + k: p[k].reshape(-1)[idx] for k in ("t", "dt", "flags", "status")},
+              "node_index": idx,
+              "counters": np.array([v for k, v in counters.items() if not k.startswith("ms_")])}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), np.ascontiguousarray(a, np.float64))
 
 
 def growing_wind(x_nodes):
@@ -521,7 +547,14 @@ def main():
     ap.add_argument("--solver", default="Tsit5", choices=["Tsit5", "DP5", "AutoTsit5"],
                     help="ODESettings.solver; AutoTsit5 = the reference's default AutoTsit5(Rosenbrock23()): the same "
                          "arithmetic as Tsit5 on this workload (the stiffness monitor never fires) plus the monitor")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed steps computed in their last step to DIR/<name>.npy (see dump_outputs; "
+                         "with N > 1 every rank writes its strip as <name>_rank<r>.npy)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the CUDA path: not with --impl reference")
     global SOLVER
     SOLVER = args.solver
     if args.warmup < 3:
@@ -556,10 +589,17 @@ def main():
         emit(line)
         return 0
 
-    # ---- our arm -------------------------------------------------------------------
+    # ---- our arm ------------------------------------------------------------------------------
+    # The library build() compiled, unless a source has changed since: then its sources are compiled into a
+    # temporary directory and that library is timed, so the numbers are always those of the sources as they stand
+    # and the tree (possibly read-only) is left as build() left it.
     import build_lib
-    if rank == 0 or world == 1:
-        build_lib.build()
+    if build_lib.needs_build():
+        import tempfile
+        from picles_b200 import _abi
+        lib_dir = tempfile.TemporaryDirectory(prefix="picles_b200_")  # removed when main() returns
+        log(f"libpicles_b200.so is missing or older than its sources: building them into {lib_dir.name}")
+        _abi.LIB_PATH = build_lib.build(out=os.path.join(lib_dir.name, "libpicles_b200.so"))
     dist = None
     affinity = None
     if world > 1:
@@ -627,6 +667,8 @@ def main():
     clocks = sampler.stop() if rank == 0 else None
     hist += eng.attempt_histogram()            # of the last timed step
     n_active = sum(c["n_active"] for c in per_step)  # particle-steps of this rank in the region
+    if args.dump_outputs:                      # before the legs below step the same engine further
+        dump_outputs(args.dump_outputs, eng, per_step[-1], DUMP_NODES // world, f"_rank{rank}" if world > 1 else "")
 
     # ---- the reference's default solver on the same workload ---------------------------------
     # ODESettings.solver defaults to AutoTsit5(Rosenbrock23()) (particle_waves_v5.jl:47).  On this
