@@ -40,7 +40,7 @@
 extern "C" {
 #endif
 
-#define PICLES_ABI_VERSION 2
+#define PICLES_ABI_VERSION 3
 
 typedef struct picles_handle picles_t;
 
@@ -174,6 +174,32 @@ int picles_abi_version(void);
 int picles_create(picles_t** h, int device_id);
 int picles_destroy(picles_t* h);
 const char* picles_last_error(picles_t* h);
+
+/* ---- ensembles: many members on one grid, stepped together ------------------------------
+ * A handle may carry `members` models that share the grid (mask, projection kernel, great-circle
+ * coefficient, boundary types) and picles_params_t; each member has its own winds, particles,
+ * deposit records and State.  All members step with the same t and dt_model in the same kernel
+ * launches: one step launches the kernels one model does, whatever the member count.
+ *
+ * Layout rule: every per-node plane argument grows from ny_local*Nx to members*ny_local*Nx values,
+ * member slowest — a plane of E members is E single-member planes back to back.  This holds for the
+ * winds of picles_seed / picles_step / picles_upload_winds / picles_set_wind_midlevels, for
+ * picles_get_state / picles_set_state (3 planes of E*ny_local*Nx), picles_get_particles,
+ * picles_get_solver_state, picles_get_fields, picles_snapshot_begin, picles_state_dev /
+ * picles_wind_dev and picles_get_row_reach (E*ny_local rows).  The grid arguments of
+ * picles_set_grid* (mask, M, pc_coef, the raw metric) and picles_get_metric stay single planes.
+ * Counters and the attempt histogram are summed over the members; reach and max_attempts are the
+ * maximum over the members; picles_state_energy_sum sums every member.
+ *
+ * With members > 1 these return PICLES_ERR_ARG: a strip cut (j0 != 0, ny_local != Ny or halo != 0),
+ * members*ny_local*Nx >= 2^31, picles_comm_init / picles_comm_destroy, picles_halo_*,
+ * picles_step_strip, the wind-mesh calls and picles_checkpoint_*.
+ */
+/* before picles_set_grid* (PICLES_ERR_STATE after it); 1..65535, default 1 */
+int picles_set_members(picles_t* h, int members);
+/* per member (members values): picles_state_energy_sum of that member's State, by the same two-stage
+   reduction, so sums[m] equals what a single-member handle with member m's State returns, bit for bit */
+int picles_member_energy_sums(picles_t* h, double* sums);
 
 /* ---- setup ------------------------------------------------------------- */
 /*

@@ -56,6 +56,8 @@ def eval_wind(f, X, Y, t):
 
 
 class WaveGrowth2D:
+    members = 1  # models stepped together on this grid (WaveGrowth2DEnsemble)
+
     def __init__(self, *, grid, winds, ODEsys, ODEvars=None, layers=1, clock=None, ODEsets=None,
                  ODEinit_type="wind_sea", minimal_particle=None, minimal_state=None, currents=None,
                  periodic_boundary=True, boundary_type="same", CBsets=None, movie=False,
@@ -140,7 +142,7 @@ class WaveGrowth2D:
             self._engine = B200Engine(self.Nx, self.Ny, g.stats.Nx.code, g.stats.Ny.code,
                                       plane(g.data.mask).astype(np.uint8), self.params, M=M, M_const=met["M_const"],
                                       pc=pc, device=self.architecture.devices[0], j0=j0, ny_local=ny, halo=halo,
-                                      metric=metric)
+                                      metric=metric, members=self.members)
             self._rows = rows
             if self._gridded_winds is not None:  # upload the wind mesh once; sampled on the device
                 self._gridded_winds.bind(self._engine, plane(g.data.x), plane(g.data.y))

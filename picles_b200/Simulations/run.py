@@ -116,7 +116,8 @@ def run(sim, store=False, pickup=False, cash_store=False, debug=False):
         nonlocal pending
         if pending is not None:
             eng.snapshot_wait()
-            sim.store.store.append(np.array(pending.transpose(2, 1, 0), copy=True))   # (Nx, Ny, 3) like model.State
+            # (3, [E,] ny, Nx) -> ([E,] Nx, Ny, 3) like model.State
+            sim.store.store.append(np.array(np.moveaxis(pending, 0, -1).swapaxes(-2, -3), copy=True))
             sim.store.iteration += 1
             pending = None
 

@@ -12,7 +12,7 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("PICLES_B200_LIB", os.path.join(HERE, "libpicles_b200.so"))
 
-ABI_VERSION = 2
+ABI_VERSION = 3
 
 # enums (include/picles_b200.h)
 BND_NONPERIODIC, BND_PERIODIC, BND_TRIPOLAR_NORTH = 0, 1, 2
@@ -114,6 +114,8 @@ SYMBOLS = {
     "picles_get_metric": (C.c_int, [_vp, _vp, _vp]),
     "picles_make_boundaries": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, C.c_int, _vp, _vp]),
     "picles_set_params": (C.c_int, [_vp, C.POINTER(PiclesParams)]),
+    "picles_set_members": (C.c_int, [_vp, C.c_int]),
+    "picles_member_energy_sums": (C.c_int, [_vp, _vp]),
     "picles_seed": (C.c_int, [_vp, _vp, _vp]),
     "picles_get_row_reach": (C.c_int, [_vp, _vp]),
     "picles_halo_rows": (C.c_int, [_vp, C.POINTER(C.c_int), C.POINTER(C.c_int)]),

@@ -66,6 +66,9 @@ struct picles_handle {
     bool have_wind_mesh = false;
     bool wm_t1_valid = false;      /* the t1 wind level was sampled from the mesh at wm_t1_time */
     double wm_t1_time = 0.0;
+    int members = 1;               /* picles_set_members: ensemble members stepped together (A.members once a grid is set) */
+    double* d_member_partial = nullptr; /* picles_member_energy_sums: ENERGY_BLOCKS partial sums per member */
+    double* h_member_partial = nullptr; /* pinned */
     void* comm = nullptr; /* ncclComm_t of the strip communicator */
     int comm_rank = -1, comm_size = 0;
     char err[512];
@@ -124,14 +127,17 @@ static int make_project_maps(picles_t* h) {
         encode = (pk_encode_tiled_fn)fn;
     }
     const DeviceArrays& A = h->A;
-    cuuint64_t dims[2] = {(cuuint64_t)A.Nx, (cuuint64_t)(A.ny + 2 * A.halo)};
-    cuuint32_t box[2] = {PR_BW, PR_BH};
-    cuuint32_t estr[2] = {1, 1};
+    /* an ensemble's planes are 3-D (Nx, ny, members): a box never reaches into the next member's rows */
+    const cuuint32_t rank = A.members > 1 ? 3 : 2;
+    cuuint64_t dims[3] = {(cuuint64_t)A.Nx, (cuuint64_t)(A.ny + 2 * A.halo), (cuuint64_t)A.members};
+    cuuint32_t box[3] = {PR_BW, PR_BH, 1};
+    cuuint32_t estr[3] = {1, 1, 1};
     for (int k = 0; k < 6; k++) {
         bool cell = (k == 5);
-        cuuint64_t stride[1] = {(cuuint64_t)A.rp * (cell ? 4 : 8)};
+        const cuuint64_t row = (cuuint64_t)A.rp * (cell ? 4 : 8);
+        cuuint64_t stride[2] = {row, row * (cuuint64_t)(A.ny + 2 * A.halo)};
         CUresult r = encode(cell ? &h->maps.cell : &h->maps.rec[k], cell ? CU_TENSOR_MAP_DATA_TYPE_INT32 : CU_TENSOR_MAP_DATA_TYPE_FLOAT64,
-                            2, cell ? (void*)A.cell : (void*)A.rec[k], dims, stride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                            rank, cell ? (void*)A.cell : (void*)A.rec[k], dims, stride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                             CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         if (r != CUDA_SUCCESS) return fail(h, PICLES_ERR_CUDA, "cuTensorMapEncodeTiled(plane %d) failed with CUresult %d", k, (int)r);
     }
@@ -151,6 +157,8 @@ static void free_grid(picles_t* h) {
     h->send_lo = h->send_hi = h->recv_lo = h->recv_hi = nullptr;
     h->reach_send = nullptr;
     h->snap = nullptr;
+    h->d_member_partial = nullptr;
+    if (h->h_member_partial) { cudaFreeHost(h->h_member_partial); h->h_member_partial = nullptr; }
     h->snap_pending = false;
     h->lag_u = h->lag_v = nullptr;
     h->steps_since_seed = 0;
@@ -282,6 +290,7 @@ int picles_destroy(picles_t* h) {
     if (h->h_counters) cudaFreeHost(h->h_counters);
     if (h->d_partial) cudaFree(h->d_partial);
     if (h->h_partial) cudaFreeHost(h->h_partial);
+    if (h->h_member_partial) cudaFreeHost(h->h_member_partial);
     for (int k = 0; k < 5; k++)
         if (h->ev[k]) cudaEventDestroy(h->ev[k]);
     for (int k = 0; k < 2; k++)
@@ -295,6 +304,34 @@ int picles_destroy(picles_t* h) {
     if (h->snap_stream) cudaStreamDestroy(h->snap_stream);
     if (h->stream) cudaStreamDestroy(h->stream);
     delete h;
+    return PICLES_OK;
+}
+
+/* refusal of the calls an ensemble does not support (strips, halo exchange, wind mesh, checkpoints) */
+static int refuse_members(picles_t* h, const char* what) {
+    if (!h) return fail(nullptr, PICLES_ERR_ARG, "null handle");
+    if (h->members > 1)
+        return fail(h, PICLES_ERR_ARG, "%s is not supported for an ensemble (%d members): %s", what, h->members,
+                    "members are stepped in one handle on one GPU, with host winds, and are not checkpointed");
+    return PICLES_OK;
+}
+#define REFUSE_MEMBERS(h, what)                    \
+    do {                                           \
+        int rm_ = refuse_members((h), (what));     \
+        if (rm_) return rm_;                       \
+    } while (0)
+
+/* particles of the handle: Nx*ny per member */
+static int64_t nodes(const picles_t* h) { return (int64_t)h->A.Nx * h->A.ny * h->A.members; }
+/* entries of rowreach: the record rows of every member */
+static int64_t record_rows(const picles_t* h) { return (int64_t)(h->A.ny + 2 * h->A.halo) * h->A.members; }
+
+int picles_set_members(picles_t* h, int members) {
+    if (!h) return fail(nullptr, PICLES_ERR_ARG, "null handle");
+    if (h->have_grid) return fail(h, PICLES_ERR_STATE, "picles_set_members must be called before picles_set_grid*");
+    /* members is a launch dimension (grid z of the gather, grid y of the per-member energy sum) */
+    if (members < 1 || members > 65535) return fail(h, PICLES_ERR_ARG, "members = %d outside 1..65535", members);
+    h->members = members;
     return PICLES_OK;
 }
 
@@ -318,6 +355,13 @@ static int set_grid_impl(picles_t* h, int Nx, int Ny, int bx, int by, int j0, in
         return fail(h, PICLES_ERR_ARG, "dx, dy, angle_dx, lat and a positive R_earth are required");
     if (halo > PH_REACH_MAX_ABI) return fail(h, PICLES_ERR_ARG, "halo %d exceeds the supported reach %d", halo, PH_REACH_MAX_ABI);
     if (ny_local != Ny && halo > ny_local) return fail(h, PICLES_ERR_ARG, "halo %d wider than the strip (%d rows)", halo, ny_local);
+    const int E = h->members;
+    if (E > 1 && (j0 != 0 || ny_local != Ny || halo != 0))
+        return fail(h, PICLES_ERR_ARG, "an ensemble (%d members) cannot be a strip: j0 = %d, ny_local = %d of %d, halo = %d; "
+                    "split the members over handles instead", E, j0, ny_local, Ny, halo);
+    if (E > 1 && (int64_t)E * Nx * ny_local >= ((int64_t)1 << 31))
+        return fail(h, PICLES_ERR_ARG, "%d members x %d x %d nodes: an ensemble holds fewer than 2^31 particles "
+                    "(the AutoTsit5 pending list stores 32-bit particle indices)", E, Nx, ny_local);
     /* `halo` rows are exchanged to begin with; the record planes of a strip hold room for the widest exchange the
        gather supports, so a step whose deposits reach further only repeats exchange + gather with more rows */
     const int halo_x = halo;
@@ -328,21 +372,23 @@ static int set_grid_impl(picles_t* h, int Nx, int Ny, int bx, int by, int j0, in
     DeviceArrays& A = h->A;
     A.Nx = Nx; A.Ny = Ny; A.bx = bx; A.by = by; A.j0 = j0; A.ny = ny_local; A.halo = halo; A.hx = halo_x;
     A.rp = (Nx + REC_PITCH_ALIGN - 1) / REC_PITCH_ALIGN * REC_PITCH_ALIGN;
-    int64_t n = (int64_t)Nx * ny_local;
-    int64_t ne = (int64_t)A.rp * (ny_local + 2 * halo);
-    for (int k = 0; k < 5; k++) DALLOC(A.z[k], n);
-    DALLOC(A.t, n); DALLOC(A.dt, n); DALLOC(A.qold, n);
-    DALLOC(A.iter, n);
-    DALLOC(A.flags, n); DALLOC(A.status, n); DALLOC(A.mask, n);
-    DALLOC(A.as, n);
-    CK(cudaMemsetAsync(A.as, 0, (size_t)n, h->stream));
-    DALLOC(A.pending, n);
-    DALLOC(A.u_t, n); DALLOC(A.v_t, n); DALLOC(A.u_t1, n); DALLOC(A.v_t1, n);
+    A.members = E;
+    int64_t n = (int64_t)Nx * ny_local; /* the grid planes */
+    const int64_t nE = n * E;           /* the particle-side planes */
+    int64_t ne = (int64_t)A.rp * (ny_local + 2 * halo) * E;
+    for (int k = 0; k < 5; k++) DALLOC(A.z[k], nE);
+    DALLOC(A.t, nE); DALLOC(A.dt, nE); DALLOC(A.qold, nE);
+    DALLOC(A.iter, nE);
+    DALLOC(A.flags, nE); DALLOC(A.status, nE); DALLOC(A.mask, n);
+    DALLOC(A.as, nE);
+    CK(cudaMemsetAsync(A.as, 0, (size_t)nE, h->stream));
+    DALLOC(A.pending, nE);
+    DALLOC(A.u_t, nE); DALLOC(A.v_t, nE); DALLOC(A.u_t1, nE); DALLOC(A.v_t1, nE);
     for (int k = 0; k < 5; k++) DALLOC(A.rec[k], ne);
     DALLOC(A.cell, ne);
-    DALLOC(A.rowreach, ny_local + 2 * halo);
-    CK(cudaMemsetAsync(A.rowreach, 0, (size_t)(ny_local + 2 * halo) * 4, h->stream));
-    for (int k = 0; k < 3; k++) DALLOC(A.S[k], n);
+    DALLOC(A.rowreach, record_rows(h));
+    CK(cudaMemsetAsync(A.rowreach, 0, (size_t)record_rows(h) * 4, h->stream));
+    for (int k = 0; k < 3; k++) DALLOC(A.S[k], nE);
     CK(cudaMemcpyAsync(A.mask, mask, (size_t)n, cudaMemcpyHostToDevice, h->stream));
     if (M) {
         for (int k = 0; k < 4; k++) {
@@ -374,8 +420,8 @@ static int set_grid_impl(picles_t* h, int Nx, int Ny, int bx, int by, int j0, in
     }
     for (int k = 0; k < 5; k++) CK(cudaMemsetAsync(A.rec[k], 0, (size_t)ne * 8, h->stream));
     launch_fill_i32(A.cell, ne, -1, h->sms, h->stream);
-    for (int k = 0; k < 3; k++) CK(cudaMemsetAsync(A.S[k], 0, (size_t)n * 8, h->stream));
-    CK(cudaMemsetAsync(A.flags, 0, (size_t)n, h->stream));
+    for (int k = 0; k < 3; k++) CK(cudaMemsetAsync(A.S[k], 0, (size_t)nE * 8, h->stream));
+    CK(cudaMemsetAsync(A.flags, 0, (size_t)nE, h->stream));
     h->halo_bytes = (int64_t)halo * A.rp * (5 * 8 + 4); /* capacity of each buffer; a message carries hx rows */
     if (halo > 0) {
         DALLOC(h->send_lo, h->halo_bytes); DALLOC(h->send_hi, h->halo_bytes);
@@ -472,7 +518,7 @@ static int need_ready(picles_t* h, bool seeded) {
 /* SeedParticle from the wind already in the t1 slots (the first step's t level, see picles_step) */
 static int seed_from_t1(picles_t* h) {
     DeviceArrays& A = h->A;
-    int64_t n = (int64_t)A.Nx * A.ny;
+    int64_t n = nodes(h);
     CK(cudaMemsetAsync(h->d_counters, 0, sizeof(DeviceCounters), h->stream));
     launch_seed(A, h->P, A.u_t1, A.v_t1, h->d_counters, h->sms, h->stream);
     CK(cudaGetLastError());
@@ -495,7 +541,7 @@ int picles_seed(picles_t* h, const double* u0, const double* v0) {
     if (rc) return rc;
     if (!u0 || !v0) return fail(h, PICLES_ERR_ARG, "picles_seed: wind arrays are required");
     DeviceArrays& A = h->A;
-    int64_t n = (int64_t)A.Nx * A.ny;
+    int64_t n = nodes(h);
     /* stage the t=0 wind in the t1 slots: the first step's t level (see picles_step) */
     CK(cudaMemcpyAsync(A.u_t1, u0, (size_t)n * 8, cudaMemcpyHostToDevice, h->stream));
     CK(cudaMemcpyAsync(A.v_t1, v0, (size_t)n * 8, cudaMemcpyHostToDevice, h->stream));
@@ -506,7 +552,7 @@ int picles_seed(picles_t* h, const double* u0, const double* v0) {
 /* intermediate wind levels of the next step (host planes -> device, consumed by the next advance) */
 static int ensure_mid_planes(picles_t* h, int n_mid) {
     DeviceArrays& A = h->A;
-    const int64_t n = (int64_t)A.Nx * A.ny;
+    const int64_t n = nodes(h);
     for (int k = 0; k < n_mid; k++) {
         if (!A.u_mid[k]) { DALLOC(A.u_mid[k], n); DALLOC(A.v_mid[k], n); }
     }
@@ -520,7 +566,7 @@ int picles_set_wind_midlevels(picles_t* h, int n_mid, const double* u_mid, const
     DeviceArrays& A = h->A;
     rc = ensure_mid_planes(h, n_mid);
     if (rc) return rc;
-    const int64_t n = (int64_t)A.Nx * A.ny;
+    const int64_t n = nodes(h);
     /* same stream as the kernels: ordered after the previous step's advance, before the next one */
     for (int k = 0; k < n_mid; k++) {
         CK(cudaMemcpyAsync(A.u_mid[k], u_mid + (int64_t)k * n, (size_t)n * 8, cudaMemcpyHostToDevice, h->stream));
@@ -535,7 +581,7 @@ int picles_upload_winds(picles_t* h, const double* u_t, const double* v_t, const
     int rc = need_ready(h, true);
     if (rc) return rc;
     DeviceArrays& A = h->A;
-    size_t bytes = (size_t)A.Nx * A.ny * 8;
+    size_t bytes = (size_t)nodes(h) * 8;
     if ((u_t == nullptr) != (v_t == nullptr) || (u_t1 == nullptr) != (v_t1 == nullptr))
         return fail(h, PICLES_ERR_ARG, "wind components must be given in pairs");
     if (u_t || u_t1) h->wm_t1_valid = false;
@@ -562,7 +608,7 @@ int picles_upload_winds(picles_t* h, const double* u_t, const double* v_t, const
 static int keep_lag_level(picles_t* h) {
     DeviceArrays& A = h->A;
     if (h->steps_since_seed != 0 || h->P.on_persist || h->n_seed_off == 0) return PICLES_OK;
-    const int64_t n = (int64_t)A.Nx * A.ny;
+    const int64_t n = nodes(h);
     if (!h->lag_u) { DALLOC(h->lag_u, n); DALLOC(h->lag_v, n); }
     CK(cudaMemcpyAsync(h->lag_u, A.u_t1, (size_t)n * 8, cudaMemcpyDeviceToDevice, h->stream));
     CK(cudaMemcpyAsync(h->lag_v, A.v_t1, (size_t)n * 8, cudaMemcpyDeviceToDevice, h->stream));
@@ -576,9 +622,9 @@ int picles_step_advance(picles_t* h, double t, double dt_model) {
     (void)t;
     if (!(dt_model > 0)) return fail(h, PICLES_ERR_ARG, "dt_model must be positive");
     CK(cudaMemsetAsync(h->d_counters, 0, sizeof(DeviceCounters), h->stream));
-    CK(cudaMemsetAsync(h->A.rowreach, 0, (size_t)(h->A.ny + 2 * h->A.halo) * 4, h->stream));
+    CK(cudaMemsetAsync(h->A.rowreach, 0, (size_t)record_rows(h) * 4, h->stream));
     CK(cudaEventRecord(h->ev[0], h->stream));
-    launch_advance(h->A, h->P, dt_model, h->d_counters, h->sms, h->stream, 0, (int64_t)h->A.Nx * h->A.ny, 0);
+    launch_advance(h->A, h->P, dt_model, h->d_counters, h->sms, h->stream, 0, nodes(h), 0);
     CK(cudaEventRecord(h->ev[1], h->stream));
     CK(cudaGetLastError());
     h->timing_valid = false;
@@ -602,7 +648,7 @@ static int begin_advance(picles_t* h, double dt_model, const double* u_t, const 
         double* tv = A.v_t; A.v_t = A.v_t1; A.v_t1 = tv;
     }
     CK(cudaMemsetAsync(h->d_counters, 0, sizeof(DeviceCounters), h->stream));
-    CK(cudaMemsetAsync(A.rowreach, 0, (size_t)(A.ny + 2 * A.halo) * 4, h->stream));
+    CK(cudaMemsetAsync(A.rowreach, 0, (size_t)record_rows(h) * 4, h->stream));
     if (u_t || u_t1) {
         /* the copy stream may only overwrite the wind planes once the compute stream is past
            every earlier kernel that read them */
@@ -681,11 +727,12 @@ static int advance_range(picles_t* h, double dt_model, const double* u_t, const 
     }
     return PICLES_OK;
 }
+/* the rows of every member: an ensemble's particle-side planes are one plane of members*ny rows */
 static int upload_and_advance(picles_t* h, double dt_model, const double* u_t, const double* v_t, const double* u_t1,
                               const double* v_t1) {
     int rc = begin_advance(h, dt_model, u_t, v_t, u_t1, v_t1);
     if (rc) return rc;
-    rc = advance_range(h, dt_model, u_t, v_t, u_t1, v_t1, 0, h->A.ny);
+    rc = advance_range(h, dt_model, u_t, v_t, u_t1, v_t1, 0, h->A.ny * h->A.members);
     if (rc) return rc;
     CK(cudaEventRecord(h->ev[1], h->stream));
     CK(cudaGetLastError());
@@ -706,6 +753,7 @@ static int64_t halo_msg_bytes(const picles_t* h) { return (int64_t)h->A.hx * h->
 
 int picles_halo_rows(picles_t* h, int* rows_exchanged, int* rows_max) {
     if (!h || !h->have_grid) return fail(h, PICLES_ERR_STATE, "grid not set");
+    REFUSE_MEMBERS(h, "picles_halo_rows");
     if (rows_exchanged) *rows_exchanged = h->A.hx;
     if (rows_max) *rows_max = h->A.halo;
     return PICLES_OK;
@@ -713,6 +761,7 @@ int picles_halo_rows(picles_t* h, int* rows_exchanged, int* rows_max) {
 
 int picles_halo_widen(picles_t* h, int rows) {
     if (!h || !h->have_grid) return fail(h, PICLES_ERR_STATE, "grid not set");
+    REFUSE_MEMBERS(h, "picles_halo_widen");
     if (rows <= h->A.hx) return PICLES_OK; /* never narrowed: rows beyond hx would keep stale records */
     if (rows > h->A.halo)
         return fail(h, PICLES_ERR_HALO, "a halo of %d rows is asked for; this strip (%d rows) can exchange at most %d", rows, h->A.ny, h->A.halo);
@@ -735,13 +784,15 @@ int picles_get_row_reach(picles_t* h, int32_t* reach_rows) {
     if (rc) return rc;
     if (!reach_rows) return fail(h, PICLES_ERR_ARG, "null output");
     const DeviceArrays& A = h->A;
-    CK(cudaMemcpyAsync(reach_rows, A.rowreach + A.halo, (size_t)A.ny * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+    /* an ensemble has no halo rows: its members' rows are back to back */
+    CK(cudaMemcpyAsync(reach_rows, A.rowreach + A.halo, (size_t)A.ny * A.members * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     return PICLES_OK;
 }
 
 int picles_halo_buffers(picles_t* h, void** send_lo, void** send_hi, void** recv_lo, void** recv_hi, int64_t* nbytes) {
     if (!h || !h->have_grid) return fail(h, PICLES_ERR_STATE, "grid not set");
+    REFUSE_MEMBERS(h, "picles_halo_buffers");
     if (send_lo) *send_lo = h->send_lo;
     if (send_hi) *send_hi = h->send_hi;
     if (recv_lo) *recv_lo = h->recv_lo;
@@ -753,6 +804,7 @@ int picles_halo_buffers(picles_t* h, void** send_lo, void** send_hi, void** recv
 int picles_halo_pack(picles_t* h) {
     int rc = need_ready(h, true);
     if (rc) return rc;
+    REFUSE_MEMBERS(h, "picles_halo_pack");
     launch_halo_pack(h->A, h->send_lo, h->send_hi, h->sms, h->stream);
     CK(cudaGetLastError());
     return PICLES_OK;
@@ -761,6 +813,7 @@ int picles_halo_pack(picles_t* h) {
 int picles_halo_unpack(picles_t* h) {
     int rc = need_ready(h, true);
     if (rc) return rc;
+    REFUSE_MEMBERS(h, "picles_halo_unpack");
     launch_halo_unpack(h->A, h->recv_lo, h->recv_hi, h->d_counters, h->sms, h->stream);
     CK(cudaGetLastError());
     return PICLES_OK;
@@ -852,7 +905,7 @@ int picles_get_state(picles_t* h, double* S) {
     int rc = need_ready(h, false);
     if (rc) return rc;
     if (!S) return fail(h, PICLES_ERR_ARG, "null output");
-    int64_t n = (int64_t)h->A.Nx * h->A.ny;
+    int64_t n = nodes(h);
     for (int k = 0; k < 3; k++) CK(cudaMemcpyAsync(S + k * n, h->A.S[k], (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     return PICLES_OK;
@@ -862,7 +915,7 @@ int picles_set_state(picles_t* h, const double* S) {
     int rc = need_ready(h, false);
     if (rc) return rc;
     if (!S) return fail(h, PICLES_ERR_ARG, "null input");
-    int64_t n = (int64_t)h->A.Nx * h->A.ny;
+    int64_t n = nodes(h);
     for (int k = 0; k < 3; k++) CK(cudaMemcpyAsync(h->A.S[k], S + k * n, (size_t)n * 8, cudaMemcpyHostToDevice, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     return PICLES_OK;
@@ -872,7 +925,7 @@ int picles_get_particles(picles_t* h, double* z, double* t, double* dt, uint8_t*
     int rc = need_ready(h, true);
     if (rc) return rc;
     const DeviceArrays& A = h->A;
-    int64_t n = (int64_t)A.Nx * A.ny;
+    int64_t n = nodes(h);
     if (z) for (int k = 0; k < 5; k++) CK(cudaMemcpyAsync(z + k * n, A.z[k], (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream));
     if (t) CK(cudaMemcpyAsync(t, A.t, (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream));
     if (dt) CK(cudaMemcpyAsync(dt, A.dt, (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream));
@@ -891,7 +944,7 @@ int picles_get_solver_state(picles_t* h, int8_t* as) {
     int rc = need_ready(h, false);
     if (rc) return rc;
     if (!as) return fail(h, PICLES_ERR_ARG, "null output");
-    CK(cudaMemcpyAsync(as, h->A.as, (size_t)h->A.Nx * h->A.ny, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(as, h->A.as, (size_t)nodes(h), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     return PICLES_OK;
 }
@@ -916,7 +969,7 @@ int picles_state_energy_sum(picles_t* h, double* sum_e) {
     int rc = need_ready(h, false);
     if (rc) return rc;
     if (!sum_e) return fail(h, PICLES_ERR_ARG, "null output");
-    int64_t n = (int64_t)h->A.Nx * h->A.ny;
+    int64_t n = nodes(h);
     launch_energy(h->A.S[0], n, h->d_partial, ENERGY_BLOCKS, h->stream);
     CK(cudaGetLastError());
     CK(cudaMemcpyAsync(h->h_partial, h->d_partial, ENERGY_BLOCKS * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
@@ -924,6 +977,28 @@ int picles_state_energy_sum(picles_t* h, double* sum_e) {
     double s = 0.0;
     for (int k = 0; k < ENERGY_BLOCKS; k++) s += h->h_partial[k];
     *sum_e = s;
+    return PICLES_OK;
+}
+
+int picles_member_energy_sums(picles_t* h, double* sums) {
+    int rc = need_ready(h, false);
+    if (rc) return rc;
+    if (!sums) return fail(h, PICLES_ERR_ARG, "null output");
+    const int E = h->A.members;
+    if (E == 1) return picles_state_energy_sum(h, sums);
+    /* the two stages of picles_state_energy_sum per member: ENERGY_BLOCKS partial sums on the device, added on the host
+       in the same order, so that sums[m] is what a single-member handle with member m's State returns */
+    if (!h->d_member_partial) DALLOC(h->d_member_partial, (int64_t)E * ENERGY_BLOCKS);
+    if (!h->h_member_partial) CK(cudaMallocHost((void**)&h->h_member_partial, (size_t)E * ENERGY_BLOCKS * sizeof(double)));
+    launch_energy_members(h->A.S[0], (int64_t)h->A.Nx * h->A.ny, E, h->d_member_partial, ENERGY_BLOCKS, h->stream);
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(h->h_member_partial, h->d_member_partial, (size_t)E * ENERGY_BLOCKS * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    for (int m = 0; m < E; m++) {
+        double s = 0.0;
+        for (int k = 0; k < ENERGY_BLOCKS; k++) s += h->h_member_partial[(int64_t)m * ENERGY_BLOCKS + k];
+        sums[m] = s;
+    }
     return PICLES_OK;
 }
 
@@ -954,7 +1029,7 @@ int picles_set_option(picles_t* h, int option, int value) {
 int picles_zero_state(picles_t* h) {
     int rc = need_ready(h, false);
     if (rc) return rc;
-    int64_t n = (int64_t)h->A.Nx * h->A.ny;
+    int64_t n = nodes(h);
     for (int k = 0; k < 3; k++) CK(cudaMemsetAsync(h->A.S[k], 0, (size_t)n * 8, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     return PICLES_OK;
@@ -1056,7 +1131,7 @@ int picles_get_fields(picles_t* h, double* Hs, double* c_x, double* c_y) {
     int rc = need_ready(h, false);
     if (rc) return rc;
     const DeviceArrays& A = h->A;
-    const int64_t n = (int64_t)A.Nx * A.ny;
+    const int64_t n = nodes(h);
     const int nout = (Hs != nullptr) + (c_x != nullptr) + (c_y != nullptr);
     if (nout == 0) return PICLES_OK;
     double* d = nullptr;
@@ -1099,7 +1174,7 @@ int picles_snapshot_begin(picles_t* h, double* S_host) {
         rc = picles_snapshot_wait(h);
         if (rc) return rc;
     }
-    const int64_t n = (int64_t)h->A.Nx * h->A.ny;
+    const int64_t n = nodes(h);
     if (!h->snap) DALLOC(h->snap, 3 * n);
     for (int k = 0; k < 3; k++)
         CK(cudaMemcpyAsync(h->snap + k * n, h->A.S[k], (size_t)n * 8, cudaMemcpyDeviceToDevice, h->stream));
@@ -1151,6 +1226,7 @@ static int64_t ckpt_bytes(const picles_t* h, bool with_lag) {
 }
 int picles_checkpoint_size(picles_t* h, int64_t* nbytes) {
     if (!h || !h->have_grid || !nbytes) return fail(h, PICLES_ERR_STATE, "grid not set");
+    REFUSE_MEMBERS(h, "picles_checkpoint_size");
     *nbytes = ckpt_bytes(h, h->A.u_lag != nullptr);
     return PICLES_OK;
 }
@@ -1179,6 +1255,7 @@ static int ckpt_planes(picles_t* h, bool with_lag, void** ptr, size_t* bytes) {
 int picles_checkpoint_save(picles_t* h, void* blob, int64_t nbytes) {
     int rc = need_ready(h, true);
     if (rc) return rc;
+    REFUSE_MEMBERS(h, "picles_checkpoint_save");
     const DeviceArrays& A = h->A;
     /* intermediate wind levels staged for the next step are not part of the blob: a run resumed from it
        would integrate that step against two levels only */
@@ -1204,6 +1281,7 @@ int picles_checkpoint_save(picles_t* h, void* blob, int64_t nbytes) {
 int picles_checkpoint_load(picles_t* h, const void* blob, int64_t nbytes) {
     int rc = need_ready(h, false);
     if (rc) return rc;
+    REFUSE_MEMBERS(h, "picles_checkpoint_load");
     if (!blob || nbytes < (int64_t)sizeof(CkptHeader)) return fail(h, PICLES_ERR_ARG, "not a checkpoint");
     CkptHeader hd;
     memcpy(&hd, blob, sizeof hd);
@@ -1260,6 +1338,7 @@ int picles_comm_unique_id(char* id128, const char* nccl_path) {
 
 int picles_comm_init(picles_t* h, const char* id128, int rank, int nranks, const char* nccl_path) {
     if (!h || !id128) return fail(h, PICLES_ERR_ARG, "null argument");
+    REFUSE_MEMBERS(h, "picles_comm_init");
     if (nranks < 1 || rank < 0 || rank >= nranks) return fail(h, PICLES_ERR_ARG, "bad rank %d of %d", rank, nranks);
     if (h->comm) return fail(h, PICLES_ERR_STATE, "communicator already initialised");
     int rc = nccl_load(h, nccl_path);
@@ -1275,6 +1354,7 @@ int picles_comm_init(picles_t* h, const char* id128, int rank, int nranks, const
 
 int picles_comm_destroy(picles_t* h) {
     if (!h) return fail(nullptr, PICLES_ERR_ARG, "null handle");
+    REFUSE_MEMBERS(h, "picles_comm_destroy");
     if (h->comm) {
         cudaSetDevice(h->device);
         cudaStreamSynchronize(h->stream);
@@ -1320,6 +1400,7 @@ static int exchange_on(picles_t* h, int lo_rank, int hi_rank, cudaStream_t st) {
 int picles_halo_exchange(picles_t* h, int lo_rank, int hi_rank) {
     int rc = need_ready(h, true);
     if (rc) return rc;
+    REFUSE_MEMBERS(h, "picles_halo_exchange");
     return exchange_on(h, lo_rank, hi_rank, h->stream);
 }
 
@@ -1348,6 +1429,7 @@ int picles_step_strip(picles_t* h, double t, double dt_model, const double* u_t,
                       const double* v_t1, int lo_rank, int hi_rank) {
     int rc = need_ready(h, true);
     if (rc) return rc;
+    REFUSE_MEMBERS(h, "picles_step_strip");
     (void)t;
     const DeviceArrays& A = h->A;
     /* boundary zones: the hb rows next to each strip edge, hb = the widest exchange the strip supports.  A particle
@@ -1432,6 +1514,7 @@ static bool strictly_increasing(const double* k, int n) {
 int picles_set_wind_mesh(picles_t* h, int nxw, int nyw, int ntw, const double* xw, const double* yw, const double* tw,
                          const double* U, const double* V, const double* node_x, const double* node_y) {
     if (!h || !h->have_grid) return fail(h, PICLES_ERR_STATE, "picles_set_grid must be called first");
+    REFUSE_MEMBERS(h, "picles_set_wind_mesh (a wind mesh)");
     if (nxw < 2 || nyw < 2 || ntw < 2) return fail(h, PICLES_ERR_ARG, "wind mesh needs at least 2 knots per axis (%d, %d, %d)", nxw, nyw, ntw);
     if (!xw || !yw || !tw || !U || !V || !node_x || !node_y) return fail(h, PICLES_ERR_ARG, "picles_set_wind_mesh: null array");
     if ((int64_t)nxw * nyw >= ((int64_t)1 << 31)) return fail(h, PICLES_ERR_ARG, "wind mesh slices are limited to 2^31 values");
@@ -1466,6 +1549,7 @@ int picles_set_wind_mesh(picles_t* h, int nxw, int nyw, int ntw, const double* x
 }
 
 int picles_sample_wind_mesh(picles_t* h, double t, double* u_out, double* v_out) {
+    if (h) REFUSE_MEMBERS(h, "picles_sample_wind_mesh (a wind mesh)");
     if (!h || !h->have_wind_mesh) return fail(h, PICLES_ERR_STATE, "picles_set_wind_mesh must be called first");
     if (!u_out || !v_out) return fail(h, PICLES_ERR_ARG, "null output");
     CK(cudaSetDevice(h->device));
@@ -1485,6 +1569,7 @@ int picles_sample_wind_mesh(picles_t* h, double t, double* u_out, double* v_out)
 /* CUDA-event time of k_wind_sample over this strip (mean of `reps` launches after one warm-up),
    written into the first intermediate-level planes: the roofline of the ingestion kernel */
 int picles_measure_wind_sample(picles_t* h, double t, int reps, double* ms_per_launch) {
+    if (h) REFUSE_MEMBERS(h, "picles_measure_wind_sample (a wind mesh)");
     if (!h || !h->have_wind_mesh) return fail(h, PICLES_ERR_STATE, "picles_set_wind_mesh must be called first");
     if (reps < 1 || !ms_per_launch) return fail(h, PICLES_ERR_ARG, "picles_measure_wind_sample: bad argument");
     CK(cudaSetDevice(h->device));
@@ -1510,6 +1595,7 @@ int picles_measure_wind_sample(picles_t* h, double t, int reps, double* ms_per_l
 int picles_seed_wind_mesh(picles_t* h, double t0) {
     int rc = need_ready(h, false);
     if (rc) return rc;
+    REFUSE_MEMBERS(h, "picles_seed_wind_mesh (a wind mesh)");
     if (!h->have_wind_mesh) return fail(h, PICLES_ERR_STATE, "picles_set_wind_mesh must be called first");
     DeviceArrays& A = h->A;
     launch_wind_sample(h->wm, (int64_t)A.Nx * A.ny, t0, A.u_t1, A.v_t1, h->sms, h->stream);
@@ -1523,6 +1609,7 @@ int picles_seed_wind_mesh(picles_t* h, double t0) {
 int picles_stage_wind_mesh(picles_t* h, double t, double dt_model, int n_mid) {
     int rc = need_ready(h, true);
     if (rc) return rc;
+    REFUSE_MEMBERS(h, "picles_stage_wind_mesh (a wind mesh)");
     if (!h->have_wind_mesh) return fail(h, PICLES_ERR_STATE, "picles_set_wind_mesh must be called first");
     if (!(dt_model > 0)) return fail(h, PICLES_ERR_ARG, "dt_model must be positive");
     if (n_mid < 0 || n_mid > PICLES_WIND_MID_MAX) return fail(h, PICLES_ERR_ARG, "n_mid = %d outside 0..%d", n_mid, PICLES_WIND_MID_MAX);
@@ -1548,6 +1635,7 @@ int picles_stage_wind_mesh(picles_t* h, double t, double dt_model, int n_mid) {
 }
 
 int picles_step_wind_mesh(picles_t* h, double t, double dt_model, int n_mid, int lo_rank, int hi_rank) {
+    REFUSE_MEMBERS(h, "picles_step_wind_mesh (a wind mesh)");
     int rc = picles_stage_wind_mesh(h, t, dt_model, n_mid);
     if (rc) return rc;
     const DeviceArrays& A = h->A;

@@ -56,6 +56,11 @@ struct DeviceArrays {
     int j0, ny, halo; /* strip: first global row (0-based), rows owned, halo rows the record planes hold on each side */
     int hx;           /* halo rows exchanged with the y-neighbours this step (<= halo; widened when the reach asks for it) */
     int rp;           /* row pitch (elements) of the record planes rec[] / cell */
+    /* ensemble (picles_set_members): `members` models share the grid planes mask, M and pc; every other plane holds
+       `members` single-member planes of ny*Nx nodes back to back (member slowest), the record planes and rowreach
+       included.  Only the ensemble instantiations of the kernels read it.  It fills the padding in front of z[]: the size
+       of the struct and the offsets of every field (and of every kernel parameter behind it) stay as they were. */
+    int members;
     double* z[5];     /* lne, c̄_x, c̄_y, x, y */
     double *t, *dt, *qold;
     int32_t* iter;
@@ -126,6 +131,8 @@ struct DeviceWindMesh {
 };
 void launch_wind_sample(const DeviceWindMesh& W, int64_t n, double t, double* u_out, double* v_out, int sms, cudaStream_t st);
 void launch_energy(const double* e, int64_t n, double* partial, int nblocks, cudaStream_t st);
+/* launch_energy for each of `members` planes of n values back to back, in one launch: partial[m*nblocks + b] */
+void launch_energy_members(const double* e, int64_t n, int members, double* partial, int nblocks, cudaStream_t st);
 void launch_halo_pack(const DeviceArrays& A, char* lo, char* hi, int sms, cudaStream_t st);
 void launch_halo_unpack(const DeviceArrays& A, const char* lo, const char* hi, DeviceCounters* dc, int sms, cudaStream_t st);
 void launch_grid_metric(int64_t n, const double* dx, const double* dy, const double* angle_dx, const double* lat,

@@ -18,6 +18,7 @@
  * results are bit-identical to the CPU oracle.
  */
 #include <cuda_runtime.h>
+#include <stddef.h>
 #include <stdint.h>
 #include <stdlib.h>
 
@@ -31,6 +32,7 @@
 namespace picles {
 
 static_assert(PH_REACH_MAX == PH_REACH_MAX_ABI, "reach limits out of sync");
+static_assert(offsetof(DeviceArrays, z) == 10 * sizeof(int), "DeviceArrays::members must stay in the padding in front of z[]");
 
 /* every kernel this library launches is counted where it is launched (bench.py reports the count of its timed region) */
 static std::atomic<long long> g_launches{0};
@@ -119,15 +121,24 @@ __device__ __forceinline__ int64_t rec_index(const DeviceArrays& A, int64_t l) {
     return (jr + A.halo) * A.rp + (l - jr * A.Nx);
 }
 
+/* node of the shared grid planes (mask, M, pc) that particle l of an ensemble lives on: l within its member.  The
+   record index and the record row stay linear in l (rec_index): members are whole blocks of rows, and an ensemble has
+   no halo rows */
+template <bool ENS>
+__device__ __forceinline__ int64_t grid_node(const DeviceArrays& A, int64_t l) {
+    return ENS ? l % ((int64_t)A.Nx * A.ny) : l;
+}
+
 /* ---- seed ------------------------------------------------------------------ */
+template <bool ENS = false>
 __global__ void __launch_bounds__(256) k_seed(DeviceArrays A, picles_params_t P, const double* __restrict__ u0,
                                               const double* __restrict__ v0, DeviceCounters* dc) {
-    int64_t n = (int64_t)A.Nx * A.ny;
+    int64_t n = ENS ? (int64_t)A.Nx * A.ny * A.members : (int64_t)A.Nx * A.ny;
     int32_t n_off = 0; /* iterated particles seeded off */
     for (int64_t l = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; l < n; l += (int64_t)gridDim.x * blockDim.x) {
         Particle p;
         double e, mx, my;
-        seed_particle(P, A.mask[l], u0[l], v0[l], p, e, mx, my);
+        seed_particle(P, A.mask[grid_node<ENS>(A, l)], u0[l], v0[l], p, e, mx, my);
         if ((p.flags & PICLES_PF_ACTIVE) && !(p.flags & PICLES_PF_ON)) n_off++;
         store_particle(A, l, p);
         A.as[l] = 0;
@@ -160,7 +171,7 @@ __global__ void __launch_bounds__(256) k_seed(DeviceArrays A, picles_params_t P,
 #else
 #define ADV_BOUNDS __launch_bounds__(ADV_THREADS, ADV_MIN_BLOCKS)
 #endif
-template <bool PER_NODE_M, bool AUTOSW, int TSIT5 = 0>
+template <bool PER_NODE_M, bool AUTOSW, int TSIT5 = 0, bool ENS = false>
 __global__ void ADV_BOUNDS
 k_advance(DeviceArrays A, picles_params_t P, double DT, DeviceCounters* dc, int64_t l_begin, int64_t l_end, int64_t l2_begin,
           int64_t l2_end, int slot) {
@@ -193,13 +204,14 @@ k_advance(DeviceArrays A, picles_params_t P, double DT, DeviceCounters* dc, int6
         const uint8_t flags = (l < lim) ? A.flags[l] : (uint8_t)0;
         if (flags & PICLES_PF_ACTIVE) { /* else: the record stays invalid (set at seed) */
             int64_t le = rec_index(A, l);
+            const int64_t g = grid_node<ENS>(A, l);
             Particle p;
             load_particle(A, l, p);
             if (AUTOSW) load_as(A, P, l, p);
             double M[4];
-            if (PER_NODE_M) { M[0] = A.M[0][l]; M[1] = A.M[1][l]; M[2] = A.M[2][l]; M[3] = A.M[3][l]; }
+            if (PER_NODE_M) { M[0] = A.M[0][g]; M[1] = A.M[1][g]; M[2] = A.M[2][g]; M[3] = A.M[3][g]; }
             else { M[0] = A.Mc[0]; M[1] = A.Mc[1]; M[2] = A.Mc[2]; M[3] = A.Mc[3]; }
-            double pc = A.pc ? A.pc[l] : 0.0;
+            double pc = A.pc ? A.pc[g] : 0.0;
             Record r;
             double um[PH_WIND_SEG_MAX], vm[PH_WIND_SEG_MAX];
 #pragma unroll
@@ -214,7 +226,7 @@ k_advance(DeviceArrays A, picles_params_t P, double DT, DeviceCounters* dc, int6
                B-1 as run never advances its own clock, so its t_end stays at 0 + DT — the level kept from the first step */
             double wu1 = A.u_t1[l], wv1 = A.v_t1[l];
             if (A.u_lag && !(flags & PICLES_PF_ON)) { wu1 = A.u_lag[l]; wv1 = A.v_lag[l]; }
-            const bool pending = advance_particle<AUTOSW, TSIT5>(P, p, A.mask[l], DT, A.u_t[l], A.v_t[l], wu1, wv1, A.n_mid, um,
+            const bool pending = advance_particle<AUTOSW, TSIT5>(P, p, A.mask[g], DT, A.u_t[l], A.v_t[l], wu1, wv1, A.n_mid, um,
                                                           vm, M, pc, r, c, K, attempts);
             if (AUTOSW && pending) {
                 /* AutoSwitch handed the particle to Rosenbrock23: park the state reached so far; the
@@ -250,7 +262,7 @@ k_advance(DeviceArrays A, picles_params_t P, double DT, DeviceCounters* dc, int6
  * indices to a list, so this kernel costs one launch when the list is empty.  One block per SM,
  * all registers: nothing here is tuned.
  */
-template <bool PER_NODE_M>
+template <bool PER_NODE_M, bool ENS = false>
 __global__ void __launch_bounds__(ADV_THREADS, 1)
 k_advance_resume(DeviceArrays A, picles_params_t P, double DT, DeviceCounters* dc, int64_t l_begin, int64_t l_end) {
     __shared__ double s_k[KS_SLOTS * ADV_THREADS];
@@ -267,11 +279,12 @@ k_advance_resume(DeviceArrays A, picles_params_t P, double DT, DeviceCounters* d
         const int64_t l = A.pending[q];
         const int64_t le = rec_index(A, l);
         if (A.cell[le] != PH_CELL_PENDING) continue;
+        const int64_t g = grid_node<ENS>(A, l);
         Particle p;
         load_particle(A, l, p);
         load_as(A, P, l, p);
         ResumeArgs R;
-        R.mask = A.mask[l]; R.nmid = A.n_mid; R.attempts = (int)A.rec[1][le];
+        R.mask = A.mask[g]; R.nmid = A.n_mid; R.attempts = (int)A.rec[1][le];
         R.DT = DT; R.t_start = A.rec[0][le];
         R.wu0 = A.u_t[l]; R.wv0 = A.v_t[l]; R.wu1 = A.u_t1[l]; R.wv1 = A.v_t1[l];
         for (int k = 0; k < PH_WIND_SEG_MAX; k++) {
@@ -279,9 +292,9 @@ k_advance_resume(DeviceArrays A, picles_params_t P, double DT, DeviceCounters* d
             R.um[k] = have ? A.u_mid[k][l] : 0.0;
             R.vm[k] = have ? A.v_mid[k][l] : 0.0;
         }
-        if (PER_NODE_M) { R.M[0] = A.M[0][l]; R.M[1] = A.M[1][l]; R.M[2] = A.M[2][l]; R.M[3] = A.M[3][l]; }
+        if (PER_NODE_M) { R.M[0] = A.M[0][g]; R.M[1] = A.M[1][g]; R.M[2] = A.M[2][g]; R.M[3] = A.M[3][g]; }
         else { R.M[0] = A.Mc[0]; R.M[1] = A.Mc[1]; R.M[2] = A.Mc[2]; R.M[3] = A.Mc[3]; }
-        R.pc = A.pc ? A.pc[l] : 0.0;
+        R.pc = A.pc ? A.pc[g] : 0.0;
         Record r;
         const int32_t max_before = c.max_attempts;
         c.max_attempts = 0;
@@ -442,11 +455,50 @@ __device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, i
                  : "memory");
 }
 
-template <int HY>
+/* the planes of ensemble member m, as a single-member DeviceArrays (no halo: every member owns whole rows) */
+__device__ __forceinline__ void member_planes(const DeviceArrays& A, int m, DeviceArrays& B) {
+    B = A;
+    const int64_t o = (int64_t)m * A.Nx * A.ny, orec = (int64_t)m * A.ny * A.rp;
+    for (int k = 0; k < 5; k++) { B.z[k] += o; B.rec[k] += orec; }
+    B.t += o; B.dt += o; B.qold += o; B.iter += o; B.flags += o; B.status += o; B.as += o;
+    B.u_t += o; B.v_t += o; B.u_t1 += o; B.v_t1 += o;
+    for (int k = 0; k < PICLES_WIND_MID_MAX; k++)
+        if (B.u_mid[k]) { B.u_mid[k] += o; B.v_mid[k] += o; }
+    if (B.u_lag) { B.u_lag += o; B.v_lag += o; }
+    for (int k = 0; k < 3; k++) B.S[k] += o;
+    B.cell += orec;
+    B.rowreach += (int64_t)m * A.ny;
+    B.members = 1;
+}
+/* the planes the gather of this block reads and writes: those of its member (blockIdx.z) in an ensemble, placed in
+   shared memory once per block */
+template <bool ENS>
+__device__ __forceinline__ const DeviceArrays& block_planes(const DeviceArrays& A) {
+    if constexpr (ENS) {
+        __shared__ DeviceArrays s_member;
+        if (threadIdx.x == 0) member_planes(A, blockIdx.z, s_member);
+        __syncthreads();
+        return s_member;
+    } else {
+        return A;
+    }
+}
+__device__ __forceinline__ void tma_load_3d(void* dst, const CUtensorMap* map, int c0, int c1, int c2, unsigned long long* mbar) {
+    asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
+                 :
+                 : "r"(smem_u32(dst)), "l"((unsigned long long)map), "r"(smem_u32(mbar)), "r"(c0), "r"(c1), "r"(c2)
+                 : "memory");
+}
+
+/* ENS: blockIdx.z is the ensemble member.  Its tiles come from 3-D tensor maps (x, row, member), so a box that sticks
+   out of the member's rows is zero-filled exactly as the 2-D box of a single model is, and no member reads another's
+   records */
+template <int HY, bool ENS = false>
 __global__ void __launch_bounds__(PR_THREADS, PR_MIN_BLOCKS)
-k_project_remesh(const __grid_constant__ ProjectMaps maps, const __grid_constant__ DeviceArrays A,
+k_project_remesh(const __grid_constant__ ProjectMaps maps, const __grid_constant__ DeviceArrays A_all,
                  const __grid_constant__ picles_params_t P, double DT, int n_classes,
                  int accumulate, DeviceCounters* dc) {
+    const DeviceArrays& A = block_planes<ENS>(A_all);
     extern __shared__ __align__(128) unsigned char pr_smem[];
     /* TMA destinations must be 128-byte aligned whatever static shared memory precedes them */
     PRTile& T = *reinterpret_cast<PRTile*>(pr_smem + ((128u - (smem_u32(pr_smem) & 127u)) & 127u));
@@ -497,9 +549,15 @@ k_project_remesh(const __grid_constant__ ProjectMaps maps, const __grid_constant
         asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(&T.mbar)), "r"(PR_TILE_BYTES)
                      : "memory");
         const int c0 = i0 - PR_HX, c1 = jr0 + A.halo - HY;
+        if constexpr (ENS) {
 #pragma unroll
-        for (int k = 0; k < 5; k++) tma_load_2d(T.rec[k], &maps.rec[k], c0, c1, &T.mbar);
-        tma_load_2d(T.cell, &maps.cell, c0, c1, &T.mbar);
+            for (int k = 0; k < 5; k++) tma_load_3d(T.rec[k], &maps.rec[k], c0, c1, blockIdx.z, &T.mbar);
+            tma_load_3d(T.cell, &maps.cell, c0, c1, blockIdx.z, &T.mbar);
+        } else {
+#pragma unroll
+            for (int k = 0; k < 5; k++) tma_load_2d(T.rec[k], &maps.rec[k], c0, c1, &T.mbar);
+            tma_load_2d(T.cell, &maps.cell, c0, c1, &T.mbar);
+        }
     }
     /* the flags of my nodes, issued while the tiles are in flight (branch A of the remesh
        needs nothing else; the wind is only read on the rare reseed / switch-off branches) */
@@ -573,7 +631,7 @@ k_project_remesh(const __grid_constant__ ProjectMaps maps, const __grid_constant
 }
 
 /* ---- energy sum (deterministic two-stage) ---------------------------------------- */
-__global__ void __launch_bounds__(256) k_energy(const double* __restrict__ e, int64_t n, double* __restrict__ partial) {
+__device__ __forceinline__ void energy_partial(const double* __restrict__ e, int64_t n, double* __restrict__ partial) {
     __shared__ double sh[256];
     double s = 0.0;
     for (int64_t l = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; l < n; l += (int64_t)gridDim.x * blockDim.x) s += e[l];
@@ -584,6 +642,13 @@ __global__ void __launch_bounds__(256) k_energy(const double* __restrict__ e, in
         __syncthreads();
     }
     if (threadIdx.x == 0) partial[blockIdx.x] = sh[0];
+}
+__global__ void __launch_bounds__(256) k_energy(const double* __restrict__ e, int64_t n, double* __restrict__ partial) {
+    energy_partial(e, n, partial);
+}
+/* an ensemble: blockIdx.y is the member, whose plane of n values is reduced exactly as k_energy reduces one model's */
+__global__ void __launch_bounds__(256) k_energy_members(const double* __restrict__ e, int64_t n, double* __restrict__ partial) {
+    energy_partial(e + blockIdx.y * n, n, partial + (int64_t)blockIdx.y * gridDim.x);
 }
 
 /* ---- halo pack / unpack: H rows of the 5 record planes + cell plane -------------- */
@@ -850,9 +915,41 @@ static int grid_for(int64_t n, int threads, int sms, int blocks_per_sm) {
 
 void launch_seed(const DeviceArrays& A, const picles_params_t& P, const double* u0, const double* v0, DeviceCounters* dc,
                  int sms, cudaStream_t st) {
-    int64_t n = (int64_t)A.Nx * A.ny;
-    k_seed<<<grid_for(n, 256, sms, 8), 256, 0, st>>>(A, P, u0, v0, dc);
+    int64_t n = (int64_t)A.Nx * A.ny * A.members;
+    if (A.members > 1) k_seed<true><<<grid_for(n, 256, sms, 8), 256, 0, st>>>(A, P, u0, v0, dc);
+    else k_seed<<<grid_for(n, 256, sms, 8), 256, 0, st>>>(A, P, u0, v0, dc);
     COUNT_LAUNCH(1);
+}
+
+/* launch_advance2 for an ensemble: the same choice of instantiation, each in its ensemble form */
+static void launch_advance_members(const DeviceArrays& A, const picles_params_t& P, double DT, DeviceCounters* dc, int sms,
+                                   cudaStream_t st, int64_t l_begin, int64_t l_end, int64_t l2_begin, int64_t l2_end,
+                                   int slot, int g, bool pn) {
+    const int64_t count = (l_end - l_begin) + (l2_end - l2_begin);
+    const bool spec = !P.nan_eest_rejects;
+#define ADV_ARGS A, P, DT, dc, l_begin, l_end, l2_begin, l2_end, slot
+    if (P.solver == PICLES_SOLVER_AUTOTSIT5) {
+        const int gr = grid_for(count, ADV_THREADS, sms, 1);
+        if (pn) {
+            if (P.propagation && spec) k_advance<true, true, 3, true><<<g, ADV_THREADS, 0, st>>>(ADV_ARGS);
+            else k_advance<true, true, 0, true><<<g, ADV_THREADS, 0, st>>>(ADV_ARGS);
+            k_advance_resume<true, true><<<gr, ADV_THREADS, 0, st>>>(A, P, DT, dc, l_begin, l_end);
+        } else {
+            if (P.propagation && spec) k_advance<false, true, 3, true><<<g, ADV_THREADS, 0, st>>>(ADV_ARGS);
+            else k_advance<false, true, 0, true><<<g, ADV_THREADS, 0, st>>>(ADV_ARGS);
+            k_advance_resume<false, true><<<gr, ADV_THREADS, 0, st>>>(A, P, DT, dc, l_begin, l_end);
+        }
+        COUNT_LAUNCH(2);
+    } else {
+        const bool ts5 = (P.solver == PICLES_SOLVER_TSIT5) && P.propagation && spec;
+        if (pn && ts5) k_advance<true, false, 1, true><<<g, ADV_THREADS, 0, st>>>(ADV_ARGS);
+        else if (pn) k_advance<true, false, 0, true><<<g, ADV_THREADS, 0, st>>>(ADV_ARGS);
+        else if (ts5) k_advance<false, false, 1, true><<<g, ADV_THREADS, 0, st>>>(ADV_ARGS);
+        else if (P.solver == PICLES_SOLVER_DP5 && P.propagation && spec) k_advance<false, false, 2, true><<<g, ADV_THREADS, 0, st>>>(ADV_ARGS);
+        else k_advance<false, false, 0, true><<<g, ADV_THREADS, 0, st>>>(ADV_ARGS);
+        COUNT_LAUNCH(1);
+    }
+#undef ADV_ARGS
 }
 
 /* particles [l_begin, l_end) and then [l2_begin, l2_end) of the strip (the whole strip: 0, Nx*ny and an empty
@@ -866,6 +963,10 @@ void launch_advance2(const DeviceArrays& A, const picles_params_t& P, double DT,
     if (count <= 0) return;
     int g = grid_for(count, ADV_THREADS, sms, ADV_MIN_BLOCKS);
     bool pn = (A.M[0] != nullptr);
+    if (A.members > 1) {
+        launch_advance_members(A, P, DT, dc, sms, st, l_begin, l_end, l2_begin, l2_end, slot, g, pn);
+        return;
+    }
     /* picles_params_t::nan_eest_rejects (a NaN error estimate rejected by 1/qmin instead of ending the integrator) lives
        in the generic instantiations only: the specialised ones keep the code they were measured with */
     const bool spec = !P.nan_eest_rejects;
@@ -906,17 +1007,23 @@ void launch_advance(const DeviceArrays& A, const picles_params_t& P, double DT, 
 
 int project_remesh_smem_bytes() { return (int)sizeof(PRTile) + 128; }
 cudaError_t project_remesh_configure() {
-    cudaError_t e = cudaFuncSetAttribute(k_project_remesh<PR_HY_NARROW>, cudaFuncAttributeMaxDynamicSharedMemorySize, project_remesh_smem_bytes());
-    if (e != cudaSuccess) return e;
-    return cudaFuncSetAttribute(k_project_remesh<PR_HY_WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, project_remesh_smem_bytes());
+    const int b = project_remesh_smem_bytes();
+    cudaError_t e = cudaFuncSetAttribute(k_project_remesh<PR_HY_NARROW>, cudaFuncAttributeMaxDynamicSharedMemorySize, b);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_project_remesh<PR_HY_WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, b);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_project_remesh<PR_HY_NARROW, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, b);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_project_remesh<PR_HY_WIDE, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, b);
+    return e;
 }
 /* wide: cut the 72 x 20 box as 12 target rows + 4 halo rows (previous step's reach was 3-4)
    instead of 16 + 2; a wrong guess only sends tiles through the generic gather */
 void launch_project_remesh(const ProjectMaps& maps, const DeviceArrays& A, const picles_params_t& P, double DT,
                            int n_classes, int accumulate, int wide, DeviceCounters* dc, cudaStream_t st) {
     const int TY = PR_BH - 2 * (wide ? PR_HY_WIDE : PR_HY_NARROW);
-    dim3 grid((A.Nx + PR_TX - 1) / PR_TX, (A.ny + TY - 1) / TY);
-    if (wide) k_project_remesh<PR_HY_WIDE><<<grid, PR_THREADS, project_remesh_smem_bytes(), st>>>(maps, A, P, DT, n_classes, accumulate, dc);
+    dim3 grid((A.Nx + PR_TX - 1) / PR_TX, (A.ny + TY - 1) / TY, A.members);
+    if (A.members > 1) {
+        if (wide) k_project_remesh<PR_HY_WIDE, true><<<grid, PR_THREADS, project_remesh_smem_bytes(), st>>>(maps, A, P, DT, n_classes, accumulate, dc);
+        else k_project_remesh<PR_HY_NARROW, true><<<grid, PR_THREADS, project_remesh_smem_bytes(), st>>>(maps, A, P, DT, n_classes, accumulate, dc);
+    } else if (wide) k_project_remesh<PR_HY_WIDE><<<grid, PR_THREADS, project_remesh_smem_bytes(), st>>>(maps, A, P, DT, n_classes, accumulate, dc);
     else k_project_remesh<PR_HY_NARROW><<<grid, PR_THREADS, project_remesh_smem_bytes(), st>>>(maps, A, P, DT, n_classes, accumulate, dc);
     COUNT_LAUNCH(1);
 }
@@ -933,6 +1040,10 @@ void launch_wind_sample(const DeviceWindMesh& W, int64_t n, double t, double* u_
 }
 void launch_energy(const double* e, int64_t n, double* partial, int nblocks, cudaStream_t st) {
     k_energy<<<nblocks, 256, 0, st>>>(e, n, partial);
+    COUNT_LAUNCH(1);
+}
+void launch_energy_members(const double* e, int64_t n, int members, double* partial, int nblocks, cudaStream_t st) {
+    k_energy_members<<<dim3(nblocks, members), 256, 0, st>>>(e, n, partial);
     COUNT_LAUNCH(1);
 }
 

@@ -20,10 +20,13 @@ def _ptr(a):
 
 class B200Engine:
     def __init__(self, Nx, Ny, bx, by, mask, params: PiclesParams, M=None, M_const=None, pc=None, device=0,
-                 j0=0, ny_local=None, halo=0, metric=None):
+                 j0=0, ny_local=None, halo=0, metric=None, members=1):
         """mask/M/pc cover the rows this strip owns: (ny_local, Nx), (4, ny_local, Nx), (ny_local, Nx).
         metric = dict(dx, dy, angle_dx, lat[, R_earth]) of (ny_local, Nx) planes: the per-node
-        kernel and great-circle coefficient are then formed on the device (picles_set_grid_metric)."""
+        kernel and great-circle coefficient are then formed on the device (picles_set_grid_metric).
+        members = E > 1: an ensemble of E models on this grid (picles_set_members), stepped together.  Every
+        per-node array then gains a member axis in front of its node axes: winds (E, ny, Nx), State (3, E, ny, Nx),
+        particle planes (5, E, ny, Nx) and (E, ny, Nx); the grid arrays above stay single planes."""
         self.lib = load_library()
         self.Nx, self.Ny = int(Nx), int(Ny)
         self.j0 = int(j0)
@@ -32,6 +35,11 @@ class B200Engine:
         self.device = int(device)
         self.h = C.c_void_p()
         self._check(self.lib.picles_create(C.byref(self.h), int(device)), None)
+        self.members = int(members)
+        # node-plane shape of every per-node array: (ny, Nx), or (E, ny, Nx) for an ensemble
+        self._nodes = (self.ny, self.Nx) if self.members == 1 else (self.members, self.ny, self.Nx)
+        if self.members != 1:
+            self._check(self.lib.picles_set_members(self.h, self.members))
         mask = np.ascontiguousarray(np.asarray(mask, np.uint8).reshape(self.ny, self.Nx))
         Mp = np.ascontiguousarray(np.asarray(M, np.float64).reshape(4, self.ny, self.Nx)) if M is not None else None
         Mc = np.ascontiguousarray(np.asarray(M_const, np.float64).reshape(4)) if M_const is not None else None
@@ -74,8 +82,8 @@ class B200Engine:
         if a is None:
             return None
         a = np.asarray(a, np.float64)
-        if a.shape != (self.ny, self.Nx):
-            a = np.broadcast_to(a, (self.ny, self.Nx))
+        if a.shape != self._nodes:
+            a = np.broadcast_to(a, self._nodes)
         return np.ascontiguousarray(a)
 
     # -- the path ------------------------------------------------------------------
@@ -194,22 +202,22 @@ class B200Engine:
 
     def row_reach(self):
         """per owned row: the largest reach (cells) of the deposits its particles wrote in the last step"""
-        r = np.empty(self.ny, np.int32)
+        r = np.empty(self._nodes[:-1], np.int32)
         self._check(self.lib.picles_get_row_reach(self.h, _ptr(r)))
         return r
 
     # -- accessors -----------------------------------------------------------------
     def state(self):
-        S = np.empty((3, self.ny, self.Nx))
+        S = np.empty((3,) + self._nodes)
         self._check(self.lib.picles_get_state(self.h, _ptr(S)))
         return S
 
     def set_state(self, S):
-        S = np.ascontiguousarray(np.asarray(S, np.float64).reshape(3, self.ny, self.Nx))
+        S = np.ascontiguousarray(np.asarray(S, np.float64).reshape((3,) + self._nodes))
         self._check(self.lib.picles_set_state(self.h, _ptr(S)))
 
     def particles(self):
-        sh = (self.ny, self.Nx)
+        sh = self._nodes
         z = np.empty((5,) + sh)
         t, dt = np.empty(sh), np.empty(sh)
         flags = np.empty(sh, np.uint8)
@@ -233,22 +241,23 @@ class B200Engine:
 
     def fields(self):
         """derived output fields on the device: dict(Hs=4*sqrt(e), c_x, c_y) of (ny, Nx)."""
-        out = [np.empty((self.ny, self.Nx)) for _ in range(3)]
+        out = [np.empty(self._nodes) for _ in range(3)]
         self._check(self.lib.picles_get_fields(self.h, *[_ptr(a) for a in out]))
         return dict(Hs=out[0], c_x=out[1], c_y=out[2])
 
     def pinned_state_buffer(self):
-        """(3, ny, Nx) float64 array in pinned host memory (freed with the engine)."""
-        nbytes = 3 * self.ny * self.Nx * 8
+        """(3, ny, Nx) (an ensemble: (3, E, ny, Nx)) float64 array in pinned host memory (freed with the engine)."""
+        size = 3 * int(np.prod(self._nodes))
+        nbytes = size * 8
         p = C.c_void_p()
         self._check(self.lib.picles_host_alloc(C.byref(p), nbytes), None)
         self._pinned = getattr(self, "_pinned", []) + [p]
-        buf = (C.c_double * (3 * self.ny * self.Nx)).from_address(p.value)
-        return np.frombuffer(buf, dtype=np.float64).reshape(3, self.ny, self.Nx)
+        buf = (C.c_double * size).from_address(p.value)
+        return np.frombuffer(buf, dtype=np.float64).reshape((3,) + self._nodes)
 
     def snapshot_begin(self, S_host):
         """start an asynchronous copy of State into S_host (3, ny, Nx); stepping may continue."""
-        assert S_host.dtype == np.float64 and S_host.flags["C_CONTIGUOUS"] and S_host.size == 3 * self.ny * self.Nx
+        assert S_host.dtype == np.float64 and S_host.flags["C_CONTIGUOUS"] and S_host.size == 3 * int(np.prod(self._nodes))
         self._check(self.lib.picles_snapshot_begin(self.h, _ptr(S_host)))
 
     def snapshot_wait(self):
@@ -285,7 +294,7 @@ class B200Engine:
     def solver_state(self):
         """AutoSwitch state per particle (AutoTsit5): run length of the stiffness test, +64 while
         Rosenbrock23 is the current algorithm"""
-        a = np.empty((self.ny, self.Nx), np.int8)
+        a = np.empty(self._nodes, np.int8)
         self._check(self.lib.picles_get_solver_state(self.h, _ptr(a)))
         return a
 
@@ -333,3 +342,9 @@ class B200Engine:
         s = C.c_double()
         self._check(self.lib.picles_state_energy_sum(self.h, C.byref(s)))
         return s.value
+
+    def member_energy_sums(self):
+        """energy_sum() of every member, (E,): bit for bit what a single-member engine with that member's State returns"""
+        s = np.empty(self.members)
+        self._check(self.lib.picles_member_energy_sums(self.h, _ptr(s)))
+        return s
