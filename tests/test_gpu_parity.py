@@ -24,14 +24,16 @@ class StripSet:
     """N strip handles on one GPU with the host-driven halo exchange a multi-GPU host
     performs (here: device-to-device copies through the C ABI)."""
 
-    def __init__(self, grid, P, nstrips, halo):
+    def __init__(self, grid, P, nstrips, halo, bounds=None):
+        """bounds: the (first, end) rows of every strip; default: nstrips strips of nearly equal height"""
         from picles_b200._abi import BND_PERIODIC
         from picles_b200.engine import B200Engine
         self.g, self.ns, self.halo = grid, nstrips, halo
         self.periodic = grid["by"] == BND_PERIODIC
         Nx, Ny = grid["Nx"], grid["Ny"]
         self.Nx, self.Ny = Nx, Ny
-        self.bounds = [(Ny * r // nstrips, Ny * (r + 1) // nstrips) for r in range(nstrips)]
+        self.bounds = bounds or [(Ny * r // nstrips, Ny * (r + 1) // nstrips) for r in range(nstrips)]
+        assert len(self.bounds) == nstrips
         self.e = []
         for a, b in self.bounds:
             M = grid["M"][:, a:b] if grid["M"] is not None else None

@@ -1,20 +1,17 @@
 """GPU (-m gpu): the randomized configurations of tests/test_independent_model.py through the CUDA path, bit for bit
 against the oracle.
 
-Written after round 2's GPU budget was spent, so this file has NEVER RUN ON A GPU.  The host build of the same device
-header is bit-exact with the oracle on 150 seeds of this generator (tests/test_device_path_cpu.py runs ten of them),
-but the CUDA path also has its fast arithmetic copies (unchecked divisions and table-driven exp where the operand
-ranges are proven, with a checked fallback), which only a GPU exercises.  Until the file has been seen green once it
-is reported, not gating: xfail(strict=False) — an `x` in the run is a finding to look at, an `X` is the expected
-result."""
+The host build of the same device header is bit-exact with the oracle on 150 seeds of this generator
+(tests/test_device_path_cpu.py runs ten of them), but the CUDA path also has its fast arithmetic copies (unchecked
+divisions and table-driven exp where the operand ranges are proven, with a checked fallback), which only a GPU
+exercises."""
 import numpy as np
 import pytest
 
 from common import compare_models, make_oracle
 from scenarios import run_pair
 
-pytestmark = [pytest.mark.gpu,
-              pytest.mark.xfail(strict=False, reason="never run on a GPU yet (round-2 GPU budget spent): reported, not gating")]
+pytestmark = pytest.mark.gpu
 
 
 @pytest.mark.parametrize("seed", range(10))
