@@ -108,6 +108,8 @@ def shim_lib():
         lib.shim_set_accumulate.argtypes = [vp, i32]
         lib.shim_set_specialised.argtypes = [i32]
         lib.shim_get_specialised.restype = i32
+        lib.shim_advance_template.restype = i32
+        lib.shim_advance_template.argtypes = [C.POINTER(PiclesParams), i32]
         lib.shim_set_wind_midlevels.argtypes = [vp, i32, vp, vp, i64]
         lib.shim_wind_mesh_sample.argtypes = [i32, i32, i32, vp, vp, vp, vp, vp, i64, vp, vp, d, vp, vp]
         lib.shim_seed.argtypes = [vp, vp, vp]
