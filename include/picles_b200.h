@@ -193,7 +193,10 @@ const char* picles_last_error(picles_t* h);
  *
  * With members > 1 these return PICLES_ERR_ARG: a strip cut (j0 != 0, ny_local != Ny or halo != 0),
  * members*ny_local*Nx >= 2^31, picles_comm_init / picles_comm_destroy, picles_halo_*,
- * picles_step_strip, the wind-mesh calls and picles_checkpoint_*.
+ * picles_step_strip, picles_set_wind_mesh (one mesh for every member) and picles_checkpoint_*; and,
+ * until picles_set_member_wind_meshes has given every member its mesh, picles_seed_wind_mesh /
+ * picles_stage_wind_mesh / picles_step_wind_mesh / picles_sample_wind_mesh /
+ * picles_measure_wind_sample.
  */
 /* before picles_set_grid* (PICLES_ERR_STATE after it); 1..65535, default 1 */
 int picles_set_members(picles_t* h, int members);
@@ -354,8 +357,24 @@ int picles_set_wind_mesh(picles_t* h, int nxw, int nyw, int ntw,
                          const double* xw, const double* yw, const double* tw,
                          const double* U, const double* V,
                          const double* node_x, const double* node_y);
-/* the mesh sampled at this strip's nodes at time t, to host (ny_local*Nx each): the values the
-   closure u.(grid.data.x, grid.data.y, t) would return */
+/* an ensemble's wind meshes, one per member on shared knots: xw, yw, tw, node_x and node_y as in
+ * picles_set_wind_mesh (node_x, node_y: one plane of ny_local*Nx, shared by the members); U and V
+ * hold members*ntw*nyw*nxw values, member slowest, each member's mesh as picles_set_wind_mesh takes
+ * it.  Checks, codes and messages as picles_set_wind_mesh, all before an old mesh is freed; the
+ * device holds 16*members*ntw*nyw*nxw bytes of mesh plus 16*members*nyw*nxw of scratch
+ * (PICLES_ERR_ALLOC names the bytes).  With one member this is picles_set_wind_mesh.  Then
+ * picles_seed_wind_mesh, picles_stage_wind_mesh, picles_step_wind_mesh, picles_sample_wind_mesh
+ * and picles_measure_wind_sample work on every member: member m's wind, and everything a step does
+ * with it, is bit for bit what a single-member handle given member m's mesh computes.  Each level
+ * is still two kernel launches, whatever the member count.  Not supported: knot vectors per member,
+ * and time slices streamed from the host (the whole time axis is resident). */
+int picles_set_member_wind_meshes(picles_t* h, int nxw, int nyw, int ntw,
+                                  const double* xw, const double* yw, const double* tw,
+                                  const double* U, const double* V,
+                                  const double* node_x, const double* node_y);
+/* the mesh sampled at this strip's nodes at time t, to host (ny_local*Nx each; an ensemble with
+   member meshes: members*ny_local*Nx each, member slowest): the values the closure
+   u.(grid.data.x, grid.data.y, t) would return */
 int picles_sample_wind_mesh(picles_t* h, double t, double* u_out, double* v_out);
 /* picles_seed with the wind of the mesh at time t0 */
 int picles_seed_wind_mesh(picles_t* h, double t0);
@@ -447,7 +466,9 @@ int picles_measure_fp64_peak(picles_t* h, double* tflops);
 int picles_selftest_math(picles_t* h, uint64_t seed, int iters, int64_t* out6);
 /* CUDA-event time per level of the wind-mesh sampling over this strip — the mesh-sized time blend
    plus the per-node kernel, as one step launches them (mean of `reps` repetitions): 32 algorithmic
-   bytes per node (coordinates in, wind out) against the HBM roofline */
+   bytes per node (coordinates in, wind out) against the HBM roofline.  With member meshes: the member
+   forms of both kernels, 48 bytes per member mesh point in the time blend and 16 per node plus 16 per
+   member and node in the sampler */
 int picles_measure_wind_sample(picles_t* h, double t, int reps, double* ms_per_launch);
 /* measured HBM copy bandwidth (read+write bytes / s) over a buffer of `mib` MiB */
 int picles_measure_hbm_copy(picles_t* h, int mib, double* gbs);

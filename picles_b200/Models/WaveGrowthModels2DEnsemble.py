@@ -8,7 +8,8 @@ share the grid, the mask, the projection kernel and every setting, and each step
 kernels one model launches, whatever E is.
 
 Layout: `State` is (E, Nx, Ny, 3) and every field of `ParticleCollection` gains a leading member
-axis; member m is exactly the `WaveGrowth2D` with `winds[m]`."""
+axis; member m is exactly the `WaveGrowth2D` with `winds[m]`.  Gridded winds (every member a
+`GriddedWinds` on the same knots) stay on the device, one mesh per member."""
 from __future__ import annotations
 
 from types import SimpleNamespace
@@ -28,29 +29,67 @@ def planes_from_state(State):
     return np.asarray(State, dtype=np.float64).transpose(3, 0, 2, 1)
 
 
+def _same_bits(a, b):
+    a, b = np.asarray(a, np.float64), np.asarray(b, np.float64)
+    return a.shape == b.shape and np.array_equal(a.view(np.uint64), b.view(np.uint64))
+
+
+class MemberGriddedWinds:
+    """The GriddedWinds of every member, on shared knots, bound to an ensemble engine as one call
+    (picles_set_member_wind_meshes): each member's mesh is then sampled on the device every step."""
+
+    def __init__(self, members):
+        self.members = list(members)
+
+    def bind(self, engine, node_x, node_y):
+        w0 = self.members[0]
+        U = np.stack([w.U for w in self.members])
+        V = np.stack([w.V for w in self.members])
+        engine.set_member_wind_meshes(w0.x, w0.y, w0.t, U, V, node_x, node_y)
+        for m, w in enumerate(self.members):
+            w._engine, w._member = engine, m
+
+
 class WaveGrowth2DEnsemble(WaveGrowth2D):
     def __init__(self, *, winds, strip=None, **kwargs):
         """The keyword constructor of WaveGrowth2D; `winds` is a list of E wind specifications, each what
-        WaveGrowth2D accepts except GriddedWinds (member m steps with winds[m])."""
+        WaveGrowth2D accepts (member m steps with winds[m]).  GriddedWinds are taken when every member has them,
+        on bitwise-identical knots: the E meshes then stay on the device and are sampled there."""
         from ..Utils.WindEmulator import GriddedWinds
         if strip is not None:
             raise ValueError("WaveGrowth2DEnsemble: strip= is not supported; split the members over models instead")
         if not isinstance(winds, (list, tuple)) or len(winds) == 0:
             raise ValueError("WaveGrowth2DEnsemble: winds must be a non-empty list with one wind specification per member")
         members = [_as_winds(w) for w in winds]
-        for m, w in enumerate(members):
-            if isinstance(w, GriddedWinds):
-                raise ValueError(f"WaveGrowth2DEnsemble: member {m} has GriddedWinds; the wind mesh is one per model, "
-                                 "give the members wind closures")
-            if not (callable(getattr(w, "u", None)) and callable(getattr(w, "v", None))):
-                raise ValueError(f"WaveGrowth2DEnsemble: member {m} needs winds u(x, y, t) and v(x, y, t)")
+        gridded = [isinstance(w, GriddedWinds) for w in members]
+        if any(gridded) and not all(gridded):
+            if gridded[0]:
+                k = gridded.index(False)
+                raise ValueError(f"WaveGrowth2DEnsemble: member 0 has GriddedWinds and member {k} has not; the members "
+                                 "take GriddedWinds on shared knots or wind closures, not both")
+            k = gridded.index(True)
+            raise ValueError(f"WaveGrowth2DEnsemble: member {k} has GriddedWinds and member 0 has not; the members "
+                             "take GriddedWinds on shared knots or wind closures, not both")
+        if all(gridded):
+            w0 = members[0]
+            for m, w in enumerate(members[1:], 1):
+                if not (_same_bits(w.x, w0.x) and _same_bits(w.y, w0.y) and _same_bits(w.t, w0.t)):
+                    raise ValueError(f"WaveGrowth2DEnsemble: member {m} has GriddedWinds on other knots than member 0; "
+                                     "the members' meshes share x, y and t")
+        else:
+            for m, w in enumerate(members):
+                if not (callable(getattr(w, "u", None)) and callable(getattr(w, "v", None))):
+                    raise ValueError(f"WaveGrowth2DEnsemble: member {m} needs winds u(x, y, t) and v(x, y, t)")
         super().__init__(winds=members[0], strip=None, **kwargs)
         self.winds = members
         self.members = len(members)
+        self._gridded_winds = MemberGriddedWinds(members) if all(gridded) else None
 
     def _wind_planes(self, t):
         """(u, v) at time t of every member, as (E, ny, Nx) C-ordered planes."""
-        self.engine  # noqa: B018  (binds self._rows)
+        eng = self.engine  # binds self._rows
+        if self._gridded_winds is not None:
+            return eng.sample_wind_mesh(t)
         X = self.grid.data.x[:, self._rows]
         Y = self.grid.data.y[:, self._rows]
         u = np.stack([eval_wind(w.u, X, Y, t).T for w in self.winds])

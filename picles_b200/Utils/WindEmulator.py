@@ -33,15 +33,19 @@ class GriddedWinds:
         self.U = np.ascontiguousarray(u.transpose(2, 1, 0))
         self.V = np.ascontiguousarray(v.transpose(2, 1, 0))
         self._engine = None
+        self._member = None  # the member this mesh drives in an ensemble engine (WaveGrowth2DEnsemble)
 
     def bind(self, engine, node_x, node_y):
         engine.set_wind_mesh(self.x, self.y, self.t, self.U, self.V, node_x, node_y)
-        self._engine = engine
+        self._engine, self._member = engine, None
 
     def _planes(self, t):
         if self._engine is None:
             raise RuntimeError("GriddedWinds is evaluated on the device: attach it to a WaveGrowth2D model first")
-        return self._engine.sample_wind_mesh(t)
+        u, v = self._engine.sample_wind_mesh(t)
+        if self._member is not None:  # the ensemble engine samples every member: this member's planes
+            return u[self._member], v[self._member]
+        return u, v
 
     # the reference's closures, on the model's own nodes
     def u(self, x, y, t):

@@ -140,6 +140,7 @@ SYMBOLS = {
     "picles_halo_exchange": (C.c_int, [_vp, C.c_int, C.c_int]),
     "picles_step_strip": (C.c_int, [_vp, C.c_double, C.c_double, _vp, _vp, _vp, _vp, C.c_int, C.c_int]),
     "picles_set_wind_mesh": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "picles_set_member_wind_meshes": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "picles_sample_wind_mesh": (C.c_int, [_vp, C.c_double, _vp, _vp]),
     "picles_seed_wind_mesh": (C.c_int, [_vp, C.c_double]),
     "picles_step_wind_mesh": (C.c_int, [_vp, C.c_double, C.c_double, C.c_int, C.c_int, C.c_int]),

@@ -64,6 +64,7 @@ struct picles_handle {
     DeviceWindMesh wm = {};        /* resident wind mesh + node coordinates (picles_set_wind_mesh) */
     std::vector<void*> wm_allocs;
     bool have_wind_mesh = false;
+    int wm_members = 1;            /* meshes resident in wm: one, or one per member (picles_set_member_wind_meshes) */
     bool wm_t1_valid = false;      /* the t1 wind level was sampled from the mesh at wm_t1_time */
     double wm_t1_time = 0.0;
     int members = 1;               /* picles_set_members: ensemble members stepped together (A.members once a grid is set) */
@@ -152,6 +153,7 @@ static void free_grid(picles_t* h) {
     for (void* p : h->wm_allocs) cudaFree(p);
     h->wm_allocs.clear();
     h->wm = DeviceWindMesh{};
+    h->wm_members = 1;
     h->have_wind_mesh = h->wm_t1_valid = false;
     memset(&h->A, 0, sizeof h->A);
     h->send_lo = h->send_hi = h->recv_lo = h->recv_hi = nullptr;
@@ -307,18 +309,31 @@ int picles_destroy(picles_t* h) {
     return PICLES_OK;
 }
 
-/* refusal of the calls an ensemble does not support (strips, halo exchange, wind mesh, checkpoints) */
+/* refusal of the calls an ensemble does not support (strips, halo exchange, checkpoints) */
 static int refuse_members(picles_t* h, const char* what) {
     if (!h) return fail(nullptr, PICLES_ERR_ARG, "null handle");
     if (h->members > 1)
         return fail(h, PICLES_ERR_ARG, "%s is not supported for an ensemble (%d members): %s", what, h->members,
-                    "members are stepped in one handle on one GPU, with host winds, and are not checkpointed");
+                    "members are stepped in one handle on one GPU and are not checkpointed");
     return PICLES_OK;
 }
 #define REFUSE_MEMBERS(h, what)                    \
     do {                                           \
         int rm_ = refuse_members((h), (what));     \
         if (rm_) return rm_;                       \
+    } while (0)
+/* the wind-mesh calls sample every member of an ensemble: each member needs its mesh (picles_set_member_wind_meshes) */
+static int refuse_members_without_meshes(picles_t* h, const char* what) {
+    if (!h) return fail(nullptr, PICLES_ERR_ARG, "null handle");
+    if (h->members > 1 && !(h->have_wind_mesh && h->wm_members == h->members))
+        return fail(h, PICLES_ERR_ARG, "%s is not supported for an ensemble (%d members) without member wind meshes: "
+                    "set one mesh per member with picles_set_member_wind_meshes", what, h->members);
+    return PICLES_OK;
+}
+#define REFUSE_MEMBERS_WITHOUT_MESHES(h, what)                  \
+    do {                                                        \
+        int rm_ = refuse_members_without_meshes((h), (what));   \
+        if (rm_) return rm_;                                    \
     } while (0)
 
 /* particles of the handle: Nx*ny per member */
@@ -1511,12 +1526,12 @@ static bool strictly_increasing(const double* k, int n) {
     }
     return true;
 }
-int picles_set_wind_mesh(picles_t* h, int nxw, int nyw, int ntw, const double* xw, const double* yw, const double* tw,
-                         const double* U, const double* V, const double* node_x, const double* node_y) {
-    if (!h || !h->have_grid) return fail(h, PICLES_ERR_STATE, "picles_set_grid must be called first");
-    REFUSE_MEMBERS(h, "picles_set_wind_mesh (a wind mesh)");
+/* `E` meshes on shared knots (E = 1: the single mesh), member slowest in U and V; every check runs before the old
+   mesh is freed */
+static int set_wind_meshes(picles_t* h, const char* what, int E, int nxw, int nyw, int ntw, const double* xw, const double* yw,
+                           const double* tw, const double* U, const double* V, const double* node_x, const double* node_y) {
     if (nxw < 2 || nyw < 2 || ntw < 2) return fail(h, PICLES_ERR_ARG, "wind mesh needs at least 2 knots per axis (%d, %d, %d)", nxw, nyw, ntw);
-    if (!xw || !yw || !tw || !U || !V || !node_x || !node_y) return fail(h, PICLES_ERR_ARG, "picles_set_wind_mesh: null array");
+    if (!xw || !yw || !tw || !U || !V || !node_x || !node_y) return fail(h, PICLES_ERR_ARG, "%s: null array", what);
     if ((int64_t)nxw * nyw >= ((int64_t)1 << 31)) return fail(h, PICLES_ERR_ARG, "wind mesh slices are limited to 2^31 values");
     if (!strictly_increasing(xw, nxw) || !strictly_increasing(yw, nyw) || !strictly_increasing(tw, ntw))
         return fail(h, PICLES_ERR_ARG, "wind mesh knot vectors must be strictly increasing");
@@ -1525,10 +1540,11 @@ int picles_set_wind_mesh(picles_t* h, int nxw, int nyw, int ntw, const double* x
     for (void* p : h->wm_allocs) cudaFree(p);
     h->wm_allocs.clear();
     h->have_wind_mesh = h->wm_t1_valid = false;
+    h->wm_members = 1;
     DeviceWindMesh& W = h->wm;
     W = DeviceWindMesh{};
     W.nx = nxw; W.ny = nyw; W.nt = ntw;
-    const int64_t n = (int64_t)h->A.Nx * h->A.ny, nm = (int64_t)nxw * nyw * ntw;
+    const int64_t n = (int64_t)h->A.Nx * h->A.ny, st = (int64_t)nxw * nyw, nm = st * ntw * E;
     int rc;
     if ((rc = wm_alloc_copy(h, &W.xw, xw, nxw)) || (rc = wm_alloc_copy(h, &W.yw, yw, nyw)) ||
         (rc = wm_alloc_copy(h, &W.tw, tw, ntw)) || (rc = wm_alloc_copy(h, &W.U, U, nm)) ||
@@ -1536,27 +1552,49 @@ int picles_set_wind_mesh(picles_t* h, int nxw, int nyw, int ntw, const double* x
         (rc = wm_alloc_copy(h, &W.node_y, node_y, n)))
         return rc;
     {
-        /* scratch of the two-pass sampler: one time-blended slice per component */
+        /* scratch of the two-pass sampler: one time-blended slice per component and member */
         void* q = nullptr;
-        const size_t nb = (size_t)nxw * nyw * 16;
+        const size_t nb = (size_t)st * E * 16;
         if (cudaMalloc(&q, nb) != cudaSuccess) return fail(h, PICLES_ERR_ALLOC, "cannot allocate %lld bytes", (long long)nb);
         h->wm_allocs.push_back(q);
-        W.Ub = (double*)q; W.Vb = W.Ub + (int64_t)nxw * nyw;
+        W.Ub = (double*)q; W.Vb = W.Ub + st * E;
     }
     CK(cudaStreamSynchronize(h->stream));
+    h->wm_members = E;
     h->have_wind_mesh = true;
     return PICLES_OK;
 }
+int picles_set_wind_mesh(picles_t* h, int nxw, int nyw, int ntw, const double* xw, const double* yw, const double* tw,
+                         const double* U, const double* V, const double* node_x, const double* node_y) {
+    if (!h || !h->have_grid) return fail(h, PICLES_ERR_STATE, "picles_set_grid must be called first");
+    if (h->members > 1)
+        return fail(h, PICLES_ERR_ARG, "picles_set_wind_mesh (one mesh) is not supported for an ensemble (%d members): "
+                    "give every member its mesh with picles_set_member_wind_meshes", h->members);
+    return set_wind_meshes(h, "picles_set_wind_mesh", 1, nxw, nyw, ntw, xw, yw, tw, U, V, node_x, node_y);
+}
+int picles_set_member_wind_meshes(picles_t* h, int nxw, int nyw, int ntw, const double* xw, const double* yw,
+                                  const double* tw, const double* U, const double* V, const double* node_x,
+                                  const double* node_y) {
+    if (!h || !h->have_grid) return fail(h, PICLES_ERR_STATE, "picles_set_grid must be called first");
+    return set_wind_meshes(h, "picles_set_member_wind_meshes", h->members, nxw, nyw, ntw, xw, yw, tw, U, V, node_x, node_y);
+}
+
+/* the wind of every member at time t at the nodes: one plane of Nx*ny values per member, member slowest */
+static void wind_sample(picles_t* h, double t, double* u_out, double* v_out) {
+    const int64_t n = (int64_t)h->A.Nx * h->A.ny;
+    if (h->wm_members > 1) launch_wind_sample_members(h->wm, h->wm_members, n, t, u_out, v_out, h->sms, h->stream);
+    else launch_wind_sample(h->wm, n, t, u_out, v_out, h->sms, h->stream);
+}
 
 int picles_sample_wind_mesh(picles_t* h, double t, double* u_out, double* v_out) {
-    if (h) REFUSE_MEMBERS(h, "picles_sample_wind_mesh (a wind mesh)");
+    if (h) REFUSE_MEMBERS_WITHOUT_MESHES(h, "picles_sample_wind_mesh (a wind mesh)");
     if (!h || !h->have_wind_mesh) return fail(h, PICLES_ERR_STATE, "picles_set_wind_mesh must be called first");
     if (!u_out || !v_out) return fail(h, PICLES_ERR_ARG, "null output");
     CK(cudaSetDevice(h->device));
-    const int64_t n = (int64_t)h->A.Nx * h->A.ny;
+    const int64_t n = nodes(h);
     double* tmp = nullptr;
     if (cudaMalloc((void**)&tmp, (size_t)n * 16) != cudaSuccess) return fail(h, PICLES_ERR_ALLOC, "cannot allocate %lld bytes", (long long)n * 16);
-    launch_wind_sample(h->wm, n, t, tmp, tmp + n, h->sms, h->stream);
+    wind_sample(h, t, tmp, tmp + n);
     cudaError_t e = cudaMemcpyAsync(u_out, tmp, (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream);
     if (e == cudaSuccess) e = cudaMemcpyAsync(v_out, tmp + n, (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
@@ -1566,21 +1604,21 @@ int picles_sample_wind_mesh(picles_t* h, double t, double* u_out, double* v_out)
     return PICLES_OK;
 }
 
-/* CUDA-event time of k_wind_sample over this strip (mean of `reps` launches after one warm-up),
-   written into the first intermediate-level planes: the roofline of the ingestion kernel */
+/* CUDA-event time of one wind level over this strip (both passes: k_wind_timeblend + k_wind_sample, or their member
+   forms; mean of `reps` launches after one warm-up), written into scratch planes of its own: the roofline of the
+   ingestion kernels */
 int picles_measure_wind_sample(picles_t* h, double t, int reps, double* ms_per_launch) {
-    if (h) REFUSE_MEMBERS(h, "picles_measure_wind_sample (a wind mesh)");
+    if (h) REFUSE_MEMBERS_WITHOUT_MESHES(h, "picles_measure_wind_sample (a wind mesh)");
     if (!h || !h->have_wind_mesh) return fail(h, PICLES_ERR_STATE, "picles_set_wind_mesh must be called first");
     if (reps < 1 || !ms_per_launch) return fail(h, PICLES_ERR_ARG, "picles_measure_wind_sample: bad argument");
     CK(cudaSetDevice(h->device));
-    DeviceArrays& A = h->A;
-    const int64_t n = (int64_t)A.Nx * A.ny;
+    const int64_t n = nodes(h);
     /* its own scratch planes: the wind levels staged for the next step are left alone */
     double* tmp = nullptr;
     if (cudaMalloc((void**)&tmp, (size_t)n * 16) != cudaSuccess) return fail(h, PICLES_ERR_ALLOC, "cannot allocate %lld bytes", (long long)n * 16);
-    launch_wind_sample(h->wm, n, t, tmp, tmp + n, h->sms, h->stream);
+    wind_sample(h, t, tmp, tmp + n);
     cudaError_t e = cudaEventRecord(h->tev[0], h->stream);
-    for (int r = 0; r < reps; r++) launch_wind_sample(h->wm, n, t, tmp, tmp + n, h->sms, h->stream);
+    for (int r = 0; r < reps; r++) wind_sample(h, t, tmp, tmp + n);
     if (e == cudaSuccess) e = cudaEventRecord(h->tev[1], h->stream);
     if (e == cudaSuccess) e = cudaEventSynchronize(h->tev[1]);
     if (e == cudaSuccess) e = cudaGetLastError();
@@ -1595,10 +1633,10 @@ int picles_measure_wind_sample(picles_t* h, double t, int reps, double* ms_per_l
 int picles_seed_wind_mesh(picles_t* h, double t0) {
     int rc = need_ready(h, false);
     if (rc) return rc;
-    REFUSE_MEMBERS(h, "picles_seed_wind_mesh (a wind mesh)");
+    REFUSE_MEMBERS_WITHOUT_MESHES(h, "picles_seed_wind_mesh (a wind mesh)");
     if (!h->have_wind_mesh) return fail(h, PICLES_ERR_STATE, "picles_set_wind_mesh must be called first");
     DeviceArrays& A = h->A;
-    launch_wind_sample(h->wm, (int64_t)A.Nx * A.ny, t0, A.u_t1, A.v_t1, h->sms, h->stream);
+    wind_sample(h, t0, A.u_t1, A.v_t1);
     h->wm_t1_valid = true;
     h->wm_t1_time = t0;
     return seed_from_t1(h);
@@ -1609,24 +1647,23 @@ int picles_seed_wind_mesh(picles_t* h, double t0) {
 int picles_stage_wind_mesh(picles_t* h, double t, double dt_model, int n_mid) {
     int rc = need_ready(h, true);
     if (rc) return rc;
-    REFUSE_MEMBERS(h, "picles_stage_wind_mesh (a wind mesh)");
+    REFUSE_MEMBERS_WITHOUT_MESHES(h, "picles_stage_wind_mesh (a wind mesh)");
     if (!h->have_wind_mesh) return fail(h, PICLES_ERR_STATE, "picles_set_wind_mesh must be called first");
     if (!(dt_model > 0)) return fail(h, PICLES_ERR_ARG, "dt_model must be positive");
     if (n_mid < 0 || n_mid > PICLES_WIND_MID_MAX) return fail(h, PICLES_ERR_ARG, "n_mid = %d outside 0..%d", n_mid, PICLES_WIND_MID_MAX);
     DeviceArrays& A = h->A;
-    const int64_t n = (int64_t)A.Nx * A.ny;
     rc = ensure_mid_planes(h, n_mid);
     if (rc) return rc;
     if (h->wm_t1_valid && h->wm_t1_time == t) { /* the previous step's t+dt level is this step's t level */
         double* tu = A.u_t; A.u_t = A.u_t1; A.u_t1 = tu;
         double* tv = A.v_t; A.v_t = A.v_t1; A.v_t1 = tv;
     } else {
-        launch_wind_sample(h->wm, n, t, A.u_t, A.v_t, h->sms, h->stream);
+        wind_sample(h, t, A.u_t, A.v_t);
     }
     const double t1 = t + dt_model;
-    launch_wind_sample(h->wm, n, t1, A.u_t1, A.v_t1, h->sms, h->stream);
+    wind_sample(h, t1, A.u_t1, A.v_t1);
     for (int k = 1; k <= n_mid; k++)
-        launch_wind_sample(h->wm, n, t + dt_model * (double)k / (double)(n_mid + 1), A.u_mid[k - 1], A.v_mid[k - 1], h->sms, h->stream);
+        wind_sample(h, t + dt_model * (double)k / (double)(n_mid + 1), A.u_mid[k - 1], A.v_mid[k - 1]);
     CK(cudaGetLastError());
     A.n_mid = n_mid;
     h->wm_t1_valid = true;
@@ -1635,7 +1672,7 @@ int picles_stage_wind_mesh(picles_t* h, double t, double dt_model, int n_mid) {
 }
 
 int picles_step_wind_mesh(picles_t* h, double t, double dt_model, int n_mid, int lo_rank, int hi_rank) {
-    REFUSE_MEMBERS(h, "picles_step_wind_mesh (a wind mesh)");
+    REFUSE_MEMBERS_WITHOUT_MESHES(h, "picles_step_wind_mesh (a wind mesh)");
     int rc = picles_stage_wind_mesh(h, t, dt_model, n_mid);
     if (rc) return rc;
     const DeviceArrays& A = h->A;

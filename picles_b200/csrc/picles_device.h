@@ -127,9 +127,14 @@ struct DeviceWindMesh {
     int nx, ny, nt;
     double *xw, *yw, *tw, *U, *V;
     double *node_x, *node_y; /* ny*Nx each */
-    double *Ub, *Vb;         /* scratch: the slice blended in time for the level being sampled, nx*ny each */
+    double *Ub, *Vb;         /* scratch: the slice blended in time for the level being sampled, nx*ny each (a slice per
+                                member with member meshes) */
 };
 void launch_wind_sample(const DeviceWindMesh& W, int64_t n, double t, double* u_out, double* v_out, int sms, cudaStream_t st);
+/* `members` meshes on W's knots (U, V: members meshes back to back; Ub, Vb: members slices), sampled at the n nodes of
+   W.node_x/node_y into members planes of n values each, member slowest */
+void launch_wind_sample_members(const DeviceWindMesh& W, int members, int64_t n, double t, double* u_out, double* v_out,
+                                int sms, cudaStream_t st);
 void launch_energy(const double* e, int64_t n, double* partial, int nblocks, cudaStream_t st);
 /* launch_energy for each of `members` planes of n values back to back, in one launch: partial[m*nblocks + b] */
 void launch_energy_members(const double* e, int64_t n, int members, double* partial, int nblocks, cudaStream_t st);

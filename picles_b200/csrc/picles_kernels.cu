@@ -905,6 +905,45 @@ __global__ void __launch_bounds__(256) k_wind_sample_x4(DeviceWindMesh D, int64_
     }
 }
 
+/* ---- an ensemble's member meshes on shared knots (picles_set_member_wind_meshes) -------------
+ * D.U, D.V hold `members` meshes back to back and D.Ub, D.Vb `members` blended slices.  The same two passes as above,
+ * each still one launch whatever the number of members. */
+/* pass 1: every member's slice at time t, blockIdx.y = member (48 B per member mesh point) */
+__global__ void __launch_bounds__(256) k_wind_timeblend_members(DeviceWindMesh D, int members, double t) {
+    WindMesh W;
+    W.nx = D.nx; W.ny = D.ny; W.nt = D.nt; W.xw = D.xw; W.yw = D.yw; W.tw = D.tw; W.U = D.U; W.V = D.V;
+    const WindMeshTime T = wm_time(W, t);
+    const int64_t st = (int64_t)D.nx * D.ny;
+    for (int m = blockIdx.y; m < members; m += gridDim.y) {
+        double* __restrict__ ub = D.Ub + st * m;
+        double* __restrict__ vb = D.Vb + st * m;
+        for (int64_t p = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; p < st; p += (int64_t)gridDim.x * blockDim.x) {
+            ub[p] = wm_timeblend_member(D.U, st, D.nt, T.it, T.dt, m, p);
+            vb[p] = wm_timeblend_member(D.V, st, D.nt, T.it, T.dt, m, p);
+        }
+    }
+}
+/* pass 2: one thread per node and chunk of WM_MEMBER_CHUNK members (blockIdx.y): the node is located once and blended
+   for each member of the chunk, its stores coalesced along the nodes of every member plane.  The member dimension fills
+   the SMs when a member has few nodes (2601 at 51 x 51). */
+#define WM_MEMBER_CHUNK 8
+__global__ void __launch_bounds__(256) k_wind_sample_members(DeviceWindMesh D, int members, int64_t n,
+                                                             double* __restrict__ u_out, double* __restrict__ v_out) {
+    WindMesh W;
+    W.nx = D.nx; W.ny = D.ny; W.nt = D.nt; W.xw = D.xw; W.yw = D.yw; W.tw = D.tw; W.U = D.U; W.V = D.V;
+    WindMeshTime T;
+    T.it = 0; T.dt = 0.0;
+    T.x0 = W.xw[0]; T.x1 = W.xw[W.nx - 1]; T.y0 = W.yw[0]; T.y1 = W.yw[W.ny - 1];
+    T.inv_hx = wm_inv_h(W.xw, W.nx); T.inv_hy = wm_inv_h(W.yw, W.ny);
+    const int m0 = blockIdx.y * WM_MEMBER_CHUNK;
+    const int m1 = (m0 + WM_MEMBER_CHUNK < members) ? m0 + WM_MEMBER_CHUNK : members;
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t l = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; l < n; l += stride) {
+        const WindMeshNode q = wm_node(W, T, __ldg(D.node_x + l), __ldg(D.node_y + l));
+        wm_sample2d_members(W, q, D.Ub, D.Vb, m0, m1, n, l, u_out, v_out);
+    }
+}
+
 /* ---- launchers ------------------------------------------------------------------ */
 static int grid_for(int64_t n, int threads, int sms, int blocks_per_sm) {
     int64_t need = (n + threads - 1) / threads;
@@ -1037,6 +1076,23 @@ void launch_wind_sample(const DeviceWindMesh& W, int64_t n, double t, double* u_
         return;
     }
     k_wind_sample<<<grid_for(n, 256, sms, 8), 256, 0, st>>>(W, n, u_out, v_out);
+}
+void launch_wind_sample_members(const DeviceWindMesh& W, int members, int64_t n, double t, double* u_out, double* v_out,
+                                int sms, cudaStream_t st) {
+    if (n <= 0) return;
+    COUNT_LAUNCH(2);
+    /* about 8 blocks per SM over both grid dimensions, at least one block per member (chunk) */
+    const int64_t cap = (int64_t)sms * 8;
+    const int64_t st_pts = (int64_t)W.nx * W.ny;
+    const int my = members < 65535 ? members : 65535;
+    int64_t bx = (cap + my - 1) / my, need = (st_pts + 255) / 256;
+    if (bx > need) bx = need;
+    k_wind_timeblend_members<<<dim3((unsigned)bx, (unsigned)my), 256, 0, st>>>(W, members, t);
+    const int chunks = (members + WM_MEMBER_CHUNK - 1) / WM_MEMBER_CHUNK;
+    bx = (cap + chunks - 1) / chunks;
+    need = (n + 255) / 256;
+    if (bx > need) bx = need;
+    k_wind_sample_members<<<dim3((unsigned)bx, (unsigned)chunks), 256, 0, st>>>(W, members, n, u_out, v_out);
 }
 void launch_energy(const double* e, int64_t n, double* partial, int nblocks, cudaStream_t st) {
     k_energy<<<nblocks, 256, 0, st>>>(e, n, partial);

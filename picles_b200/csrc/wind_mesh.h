@@ -13,7 +13,7 @@
  *     weights (1-dx, dx); the value is the nested weighted sum with the first axis outermost.
  *
  * `__host__ __device__` so tests/ can run the same code on the CPU against the CPU checker's own
- * restatement of the rule; the product only calls it from k_wind_sample.  Build rules as physics.h (no contraction; nothing here needs an fma).
+ * restatement of the rule; the product only calls it from the wind kernels.  Build rules as physics.h (no contraction; nothing here needs an fma).
  */
 #ifndef PICLES_WIND_MESH_H
 #define PICLES_WIND_MESH_H
@@ -173,6 +173,49 @@ PM_HD void wm_sample2d_x4(const WindMesh& W, const WindMeshTime& T, const double
         const int off = ix + W.nx * iy;
         u[k] = wm_blend2d(Ub + off, W.nx, dx, dy);
         v[k] = wm_blend2d(Vb + off, W.nx, dx, dy);
+    }
+}
+
+/* ---- E member meshes on shared knots (k_wind_timeblend_members, k_wind_sample_members) -----
+   An ensemble's meshes share xw, yw, tw and the node coordinates; U and V hold E meshes back to
+   back, member slowest, and the time-blended scratch holds E slices of nx*ny points.  The time
+   interval and weight are the same for every member, and a node's (ix, dx, iy, dy) does not depend
+   on the member: it is located once and blended for each member with wm_blend2d, the expression
+   wm_sample2d uses, so member m gets exactly what a single mesh made of member m's data gives. */
+struct WindMeshNode {
+    int off; /* ix + nx*iy */
+    double dx, dy;
+};
+PM_HD WindMeshNode wm_node(const WindMesh& W, const WindMeshTime& T, double x, double y) {
+    const double xp = wm_periodic(x, T.x0, T.x1);
+    const double yp = wm_periodic(y, T.y0, T.y1);
+    int ix, iy;
+    WindMeshNode q;
+    wm_locate(W.xw, W.nx, xp, T.inv_hx, ix, q.dx);
+    wm_locate(W.yw, W.ny, yp, T.inv_hy, iy, q.dy);
+    q.off = ix + W.nx * iy;
+    return q;
+}
+/* pass 1 of member m at mesh point p (slice = nx*ny): member m's slice of the scratch */
+PM_HD double wm_timeblend_member(const double* __restrict__ A, int64_t slice, int nt, int it, double dt, int m, int64_t p) {
+    return wm_timeblend(A + (int64_t)m * nt * slice, slice, it, dt, p);
+}
+/* pass 2 for node l and members [m0, m1): u_out[m*n + l], v_out[m*n + l] (the layout of every
+   per-node plane of an ensemble), so the stores of consecutive nodes stay consecutive per member */
+PM_HD void wm_sample2d_members(const WindMesh& W, const WindMeshNode& q, const double* __restrict__ Ub,
+                               const double* __restrict__ Vb, int m0, int m1, int64_t n, int64_t l,
+                               double* __restrict__ u_out, double* __restrict__ v_out) {
+    const int64_t slice = (int64_t)W.nx * W.ny;
+    for (int m = m0; m < m1; m++) {
+        const double u = wm_blend2d(Ub + slice * m + q.off, W.nx, q.dx, q.dy);
+        const double v = wm_blend2d(Vb + slice * m + q.off, W.nx, q.dx, q.dy);
+#if defined(__CUDA_ARCH__)
+        __stcs(u_out + n * m + l, u);
+        __stcs(v_out + n * m + l, v);
+#else
+        u_out[n * m + l] = u;
+        v_out[n * m + l] = v;
+#endif
     }
 }
 

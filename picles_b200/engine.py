@@ -120,8 +120,24 @@ class B200Engine:
         self._check(self.lib.picles_set_wind_mesh(self.h, xw.size, yw.size, tw.size, _ptr(xw), _ptr(yw), _ptr(tw),
                                                   _ptr(U), _ptr(V), _ptr(nx_), _ptr(ny_)))
 
+    def set_member_wind_meshes(self, xw, yw, tw, U, V, node_x, node_y):
+        """an ensemble's wind meshes, one per member on shared knots (picles_set_member_wind_meshes).
+        U, V: (E, nt, ny_w, nx_w), member m's mesh as set_wind_mesh takes it; node_x, node_y: (ny, Nx), shared by
+        the members.  seed/stage/step_wind_mesh and sample_wind_mesh then sample every member on the device."""
+        f = lambda a: np.ascontiguousarray(np.asarray(a, np.float64))
+        xw, yw, tw, U, V = f(xw), f(yw), f(tw), f(U), f(V)
+        shape = (self.members, tw.size, yw.size, xw.size)
+        if U.shape != shape or V.shape != shape:
+            raise ValueError(f"U, V must have shape (E, nt, ny, nx) = {shape}, not {U.shape} and {V.shape}")
+        plane = lambda a: np.ascontiguousarray(np.broadcast_to(np.asarray(a, np.float64), (self.ny, self.Nx)))
+        nx_, ny_ = plane(node_x), plane(node_y)
+        self._check(self.lib.picles_set_member_wind_meshes(self.h, xw.size, yw.size, tw.size, _ptr(xw), _ptr(yw),
+                                                           _ptr(tw), _ptr(U), _ptr(V), _ptr(nx_), _ptr(ny_)))
+
     def sample_wind_mesh(self, t):
-        u, v = np.empty((self.ny, self.Nx)), np.empty((self.ny, self.Nx))
+        """(u, v) of the mesh at this strip's nodes at time t: (ny, Nx) each, or (E, ny, Nx) on an ensemble"""
+        # an ensemble with member meshes writes E planes: the buffers are sized for them before the call
+        u, v = np.empty(self._nodes), np.empty(self._nodes)
         self._check(self.lib.picles_sample_wind_mesh(self.h, float(t), _ptr(u), _ptr(v)))
         return u, v
 
@@ -333,7 +349,7 @@ class B200Engine:
         return v.value
 
     def measure_wind_sample(self, t=0.0, reps=20):
-        """ms per launch of k_wind_sample over this strip (CUDA events)"""
+        """ms per wind level (time blend + sampler, or their member forms) over this strip (CUDA events)"""
         v = C.c_double()
         self._check(self.lib.picles_measure_wind_sample(self.h, float(t), int(reps), C.byref(v)))
         return v.value
