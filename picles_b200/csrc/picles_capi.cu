@@ -113,8 +113,9 @@ static int dalloc(picles_t* h, T** p, int64_t count) {
 
 /* ---- TMA tensor maps of the record planes --------------------------------------------
  * cuTensorMapEncodeTiled is a driver entry point; it is resolved through the runtime so the
- * library does not link libcuda.  Planes are 2-D (Nx, ny + 2*halo) with row pitch rp; the box
- * is the projection tile (PR_BW x PR_BH); out-of-bounds elements are zero-filled. */
+ * library does not link libcuda.  Planes are 3-D (Nx, ny + 2*halo, members) with row pitch rp; the box
+ * is the projection tile (PR_BW x PR_BH) of one member, so it never reaches into the next member's rows;
+ * out-of-bounds elements are zero-filled. */
 typedef CUresult (*pk_encode_tiled_fn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                        const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                        CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -128,8 +129,6 @@ static int make_project_maps(picles_t* h) {
         encode = (pk_encode_tiled_fn)fn;
     }
     const DeviceArrays& A = h->A;
-    /* an ensemble's planes are 3-D (Nx, ny, members): a box never reaches into the next member's rows */
-    const cuuint32_t rank = A.members > 1 ? 3 : 2;
     cuuint64_t dims[3] = {(cuuint64_t)A.Nx, (cuuint64_t)(A.ny + 2 * A.halo), (cuuint64_t)A.members};
     cuuint32_t box[3] = {PR_BW, PR_BH, 1};
     cuuint32_t estr[3] = {1, 1, 1};
@@ -138,7 +137,7 @@ static int make_project_maps(picles_t* h) {
         const cuuint64_t row = (cuuint64_t)A.rp * (cell ? 4 : 8);
         cuuint64_t stride[2] = {row, row * (cuuint64_t)(A.ny + 2 * A.halo)};
         CUresult r = encode(cell ? &h->maps.cell : &h->maps.rec[k], cell ? CU_TENSOR_MAP_DATA_TYPE_INT32 : CU_TENSOR_MAP_DATA_TYPE_FLOAT64,
-                            rank, cell ? (void*)A.cell : (void*)A.rec[k], dims, stride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                            3, cell ? (void*)A.cell : (void*)A.rec[k], dims, stride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                             CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         if (r != CUDA_SUCCESS) return fail(h, PICLES_ERR_CUDA, "cuTensorMapEncodeTiled(plane %d) failed with CUresult %d", k, (int)r);
     }
@@ -980,41 +979,38 @@ int picles_get_attempt_histogram(picles_t* h, int64_t* hist, int nbins) {
 
 int64_t picles_launch_count(void) { return (int64_t)launch_count(); }
 
+/* the energy sum of each of `groups` planes of n values of State[0], back to back, by a deterministic two-stage
+   reduction: ENERGY_BLOCKS partial sums per plane on the device (d_part), added on the host in block order (h_part) */
+static int energy_sums(picles_t* h, int64_t n, int groups, double* d_part, double* h_part, double* sums) {
+    launch_energy(h->A.S[0], n, groups, d_part, ENERGY_BLOCKS, h->stream);
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(h_part, d_part, (size_t)groups * ENERGY_BLOCKS * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    for (int m = 0; m < groups; m++) {
+        double s = 0.0;
+        for (int k = 0; k < ENERGY_BLOCKS; k++) s += h_part[(int64_t)m * ENERGY_BLOCKS + k];
+        sums[m] = s;
+    }
+    return PICLES_OK;
+}
+
 int picles_state_energy_sum(picles_t* h, double* sum_e) {
     int rc = need_ready(h, false);
     if (rc) return rc;
     if (!sum_e) return fail(h, PICLES_ERR_ARG, "null output");
-    int64_t n = nodes(h);
-    launch_energy(h->A.S[0], n, h->d_partial, ENERGY_BLOCKS, h->stream);
-    CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(h->h_partial, h->d_partial, ENERGY_BLOCKS * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
-    double s = 0.0;
-    for (int k = 0; k < ENERGY_BLOCKS; k++) s += h->h_partial[k];
-    *sum_e = s;
-    return PICLES_OK;
+    return energy_sums(h, nodes(h), 1, h->d_partial, h->h_partial, sum_e);
 }
 
 int picles_member_energy_sums(picles_t* h, double* sums) {
     int rc = need_ready(h, false);
     if (rc) return rc;
     if (!sums) return fail(h, PICLES_ERR_ARG, "null output");
+    /* each member's plane is reduced as picles_state_energy_sum reduces a single model's, so that sums[m] is what a
+       single-member handle with member m's State returns */
     const int E = h->A.members;
-    if (E == 1) return picles_state_energy_sum(h, sums);
-    /* the two stages of picles_state_energy_sum per member: ENERGY_BLOCKS partial sums on the device, added on the host
-       in the same order, so that sums[m] is what a single-member handle with member m's State returns */
     if (!h->d_member_partial) DALLOC(h->d_member_partial, (int64_t)E * ENERGY_BLOCKS);
     if (!h->h_member_partial) CK(cudaMallocHost((void**)&h->h_member_partial, (size_t)E * ENERGY_BLOCKS * sizeof(double)));
-    launch_energy_members(h->A.S[0], (int64_t)h->A.Nx * h->A.ny, E, h->d_member_partial, ENERGY_BLOCKS, h->stream);
-    CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(h->h_member_partial, h->d_member_partial, (size_t)E * ENERGY_BLOCKS * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-    CK(cudaStreamSynchronize(h->stream));
-    for (int m = 0; m < E; m++) {
-        double s = 0.0;
-        for (int k = 0; k < ENERGY_BLOCKS; k++) s += h->h_member_partial[(int64_t)m * ENERGY_BLOCKS + k];
-        sums[m] = s;
-    }
-    return PICLES_OK;
+    return energy_sums(h, (int64_t)h->A.Nx * h->A.ny, E, h->d_member_partial, h->h_member_partial, sums);
 }
 
 int picles_state_dev(picles_t* h, double** S_dev) {

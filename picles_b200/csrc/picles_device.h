@@ -58,8 +58,8 @@ struct DeviceArrays {
     int rp;           /* row pitch (elements) of the record planes rec[] / cell */
     /* ensemble (picles_set_members): `members` models share the grid planes mask, M and pc; every other plane holds
        `members` single-member planes of ny*Nx nodes back to back (member slowest), the record planes and rowreach
-       included.  Only the ensemble instantiations of the kernels read it.  It fills the padding in front of z[]: the size
-       of the struct and the offsets of every field (and of every kernel parameter behind it) stay as they were. */
+       included.  1 for a single model.  Read by k_seed and by the ensemble forms of k_advance, k_advance_resume and
+       k_project_remesh, which the launchers pick when it is above 1. */
     int members;
     double* z[5];     /* lne, c̄_x, c̄_y, x, y */
     double *t, *dt, *qold;
@@ -113,7 +113,7 @@ void launch_advance2(const DeviceArrays& A, const picles_params_t& P, double DT,
 void launch_reach_word(const int32_t* src, int32_t* dst, cudaStream_t st);
 /* kernels launched by this library since it was loaded (every launch_* call counts its kernels) */
 long long launch_count();
-/* TMA tensor maps of the six record planes (box PR_BW x PR_BH) */
+/* TMA tensor maps of the six record planes (box PR_BW x PR_BH x 1 member) */
 struct ProjectMaps {
     CUtensorMap rec[5];
     CUtensorMap cell;
@@ -135,9 +135,8 @@ void launch_wind_sample(const DeviceWindMesh& W, int64_t n, double t, double* u_
    W.node_x/node_y into members planes of n values each, member slowest */
 void launch_wind_sample_members(const DeviceWindMesh& W, int members, int64_t n, double t, double* u_out, double* v_out,
                                 int sms, cudaStream_t st);
-void launch_energy(const double* e, int64_t n, double* partial, int nblocks, cudaStream_t st);
-/* launch_energy for each of `members` planes of n values back to back, in one launch: partial[m*nblocks + b] */
-void launch_energy_members(const double* e, int64_t n, int members, double* partial, int nblocks, cudaStream_t st);
+/* nblocks partial sums of each of `members` planes of n values back to back, in one launch: partial[m*nblocks + b] */
+void launch_energy(const double* e, int64_t n, int members, double* partial, int nblocks, cudaStream_t st);
 void launch_halo_pack(const DeviceArrays& A, char* lo, char* hi, int sms, cudaStream_t st);
 void launch_halo_unpack(const DeviceArrays& A, const char* lo, const char* hi, DeviceCounters* dc, int sms, cudaStream_t st);
 void launch_grid_metric(int64_t n, const double* dx, const double* dy, const double* angle_dx, const double* lat,

@@ -6,7 +6,7 @@
  *   k_project_remesh  ParticleToNode! as a deterministic gather   (mapping_2D.jl:59-73,
  *                     over TMA-staged record tiles, fused with     ParticleInCell.jl:341-538)
  *                     remesh!/NodeToParticle!                     (mapping_2D.jl:250-356)  HBM-bound
- *   k_energy    sum of State[:,:,1]                               (run.jl:23-25)
+ *   k_energy_members  sum of State[:,:,1], per member            (run.jl:23-25)
  *
  * Layout in HBM (one y-strip per GPU): every per-node quantity is its own plane of
  * ny*Nx doubles with i (x) fastest — the memory order of the reference's column-major
@@ -32,7 +32,6 @@
 namespace picles {
 
 static_assert(PH_REACH_MAX == PH_REACH_MAX_ABI, "reach limits out of sync");
-static_assert(offsetof(DeviceArrays, z) == 10 * sizeof(int), "DeviceArrays::members must stay in the padding in front of z[]");
 
 /* every kernel this library launches is counted where it is launched (bench.py reports the count of its timed region) */
 static std::atomic<long long> g_launches{0};
@@ -121,24 +120,23 @@ __device__ __forceinline__ int64_t rec_index(const DeviceArrays& A, int64_t l) {
     return (jr + A.halo) * A.rp + (l - jr * A.Nx);
 }
 
-/* node of the shared grid planes (mask, M, pc) that particle l of an ensemble lives on: l within its member.  The
-   record index and the record row stay linear in l (rec_index): members are whole blocks of rows, and an ensemble has
-   no halo rows */
+/* node of the shared grid planes (mask, M, pc) that particle l lives on: l within its member under ENS, l itself for
+   a single model (strips included).  The record index and the record row stay linear in l (rec_index): members are
+   whole blocks of rows, and an ensemble has no halo rows */
 template <bool ENS>
 __device__ __forceinline__ int64_t grid_node(const DeviceArrays& A, int64_t l) {
     return ENS ? l % ((int64_t)A.Nx * A.ny) : l;
 }
 
 /* ---- seed ------------------------------------------------------------------ */
-template <bool ENS = false>
 __global__ void __launch_bounds__(256) k_seed(DeviceArrays A, picles_params_t P, const double* __restrict__ u0,
                                               const double* __restrict__ v0, DeviceCounters* dc) {
-    int64_t n = ENS ? (int64_t)A.Nx * A.ny * A.members : (int64_t)A.Nx * A.ny;
+    int64_t n = (int64_t)A.Nx * A.ny * A.members;
     int32_t n_off = 0; /* iterated particles seeded off */
     for (int64_t l = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; l < n; l += (int64_t)gridDim.x * blockDim.x) {
         Particle p;
         double e, mx, my;
-        seed_particle(P, A.mask[grid_node<ENS>(A, l)], u0[l], v0[l], p, e, mx, my);
+        seed_particle(P, A.mask[grid_node<true>(A, l)], u0[l], v0[l], p, e, mx, my);
         if ((p.flags & PICLES_PF_ACTIVE) && !(p.flags & PICLES_PF_ON)) n_off++;
         store_particle(A, l, p);
         A.as[l] = 0;
@@ -321,7 +319,7 @@ k_advance_resume(DeviceArrays A, picles_params_t P, double DT, DeviceCounters* d
 /* ---- projection gather + remesh ---------------------------------------------------- */
 /*
  * One block per tile of PR_TX x TY target nodes (TY = PR_BH - 2*HY).  One thread arms an mbarrier and issues
- * six TMA tile loads (cp.async.bulk.tensor.2d): the five record planes and the cell plane
+ * six TMA tile loads (cp.async.bulk.tensor.3d): the five record planes and the cell plane of its member
  * over the targets plus a halo of PR_HX x HY cells.  Boxes that stick out of the planes are
  * zero-filled by the TMA unit; a zero cell decodes to an offset that never matches, i.e.
  * "no deposit", which is exactly what lies beyond a non-periodic edge.  While the tiles are in
@@ -448,14 +446,9 @@ __device__ __noinline__ int4 cold_nodes(const DeviceArrays* Ap, const picles_par
 }
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, int c0, int c1, unsigned long long* mbar) {
-    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-                 :
-                 : "r"(smem_u32(dst)), "l"((unsigned long long)map), "r"(smem_u32(mbar)), "r"(c0), "r"(c1)
-                 : "memory");
-}
 
-/* the planes of ensemble member m, as a single-member DeviceArrays (no halo: every member owns whole rows) */
+/* the planes of ensemble member m, as a single-member DeviceArrays (an ensemble has no halo rows: every member owns
+   whole rows; member 0 is the handle's own planes, a strip's halo rows included) */
 __device__ __forceinline__ void member_planes(const DeviceArrays& A, int m, DeviceArrays& B) {
     B = A;
     const int64_t o = (int64_t)m * A.Nx * A.ny, orec = (int64_t)m * A.ny * A.rp;
@@ -471,7 +464,8 @@ __device__ __forceinline__ void member_planes(const DeviceArrays& A, int m, Devi
     B.members = 1;
 }
 /* the planes the gather of this block reads and writes: those of its member (blockIdx.z) in an ensemble, placed in
-   shared memory once per block */
+   shared memory once per block.  A single model reads its own from the kernel parameter: the copy in shared memory
+   costs it 8-10 % of the gather (measured at 4096^2) */
 template <bool ENS>
 __device__ __forceinline__ const DeviceArrays& block_planes(const DeviceArrays& A) {
     if constexpr (ENS) {
@@ -490,9 +484,9 @@ __device__ __forceinline__ void tma_load_3d(void* dst, const CUtensorMap* map, i
                  : "memory");
 }
 
-/* ENS: blockIdx.z is the ensemble member.  Its tiles come from 3-D tensor maps (x, row, member), so a box that sticks
-   out of the member's rows is zero-filled exactly as the 2-D box of a single model is, and no member reads another's
-   records */
+/* blockIdx.z is the ensemble member (0 for a single model).  Its tiles come from 3-D tensor maps (x, row, member), so
+   a box that sticks out of the member's rows is zero-filled as it is beyond a single model's edge, and no member reads
+   another's records.  ENS: more than one member (block_planes) */
 template <int HY, bool ENS = false>
 __global__ void __launch_bounds__(PR_THREADS, PR_MIN_BLOCKS)
 k_project_remesh(const __grid_constant__ ProjectMaps maps, const __grid_constant__ DeviceArrays A_all,
@@ -549,15 +543,9 @@ k_project_remesh(const __grid_constant__ ProjectMaps maps, const __grid_constant
         asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(&T.mbar)), "r"(PR_TILE_BYTES)
                      : "memory");
         const int c0 = i0 - PR_HX, c1 = jr0 + A.halo - HY;
-        if constexpr (ENS) {
 #pragma unroll
-            for (int k = 0; k < 5; k++) tma_load_3d(T.rec[k], &maps.rec[k], c0, c1, blockIdx.z, &T.mbar);
-            tma_load_3d(T.cell, &maps.cell, c0, c1, blockIdx.z, &T.mbar);
-        } else {
-#pragma unroll
-            for (int k = 0; k < 5; k++) tma_load_2d(T.rec[k], &maps.rec[k], c0, c1, &T.mbar);
-            tma_load_2d(T.cell, &maps.cell, c0, c1, &T.mbar);
-        }
+        for (int k = 0; k < 5; k++) tma_load_3d(T.rec[k], &maps.rec[k], c0, c1, blockIdx.z, &T.mbar);
+        tma_load_3d(T.cell, &maps.cell, c0, c1, blockIdx.z, &T.mbar);
     }
     /* the flags of my nodes, issued while the tiles are in flight (branch A of the remesh
        needs nothing else; the wind is only read on the rare reseed / switch-off branches) */
@@ -643,10 +631,7 @@ __device__ __forceinline__ void energy_partial(const double* __restrict__ e, int
     }
     if (threadIdx.x == 0) partial[blockIdx.x] = sh[0];
 }
-__global__ void __launch_bounds__(256) k_energy(const double* __restrict__ e, int64_t n, double* __restrict__ partial) {
-    energy_partial(e, n, partial);
-}
-/* an ensemble: blockIdx.y is the member, whose plane of n values is reduced exactly as k_energy reduces one model's */
+/* blockIdx.y is the member, whose plane of n values is reduced by the same blocks in the same order whatever gridDim.y is */
 __global__ void __launch_bounds__(256) k_energy_members(const double* __restrict__ e, int64_t n, double* __restrict__ partial) {
     energy_partial(e + blockIdx.y * n, n, partial + (int64_t)blockIdx.y * gridDim.x);
 }
@@ -955,8 +940,7 @@ static int grid_for(int64_t n, int threads, int sms, int blocks_per_sm) {
 void launch_seed(const DeviceArrays& A, const picles_params_t& P, const double* u0, const double* v0, DeviceCounters* dc,
                  int sms, cudaStream_t st) {
     int64_t n = (int64_t)A.Nx * A.ny * A.members;
-    if (A.members > 1) k_seed<true><<<grid_for(n, 256, sms, 8), 256, 0, st>>>(A, P, u0, v0, dc);
-    else k_seed<<<grid_for(n, 256, sms, 8), 256, 0, st>>>(A, P, u0, v0, dc);
+    k_seed<<<grid_for(n, 256, sms, 8), 256, 0, st>>>(A, P, u0, v0, dc);
     COUNT_LAUNCH(1);
 }
 
@@ -1094,11 +1078,7 @@ void launch_wind_sample_members(const DeviceWindMesh& W, int members, int64_t n,
     if (bx > need) bx = need;
     k_wind_sample_members<<<dim3((unsigned)bx, (unsigned)chunks), 256, 0, st>>>(W, members, n, u_out, v_out);
 }
-void launch_energy(const double* e, int64_t n, double* partial, int nblocks, cudaStream_t st) {
-    k_energy<<<nblocks, 256, 0, st>>>(e, n, partial);
-    COUNT_LAUNCH(1);
-}
-void launch_energy_members(const double* e, int64_t n, int members, double* partial, int nblocks, cudaStream_t st) {
+void launch_energy(const double* e, int64_t n, int members, double* partial, int nblocks, cudaStream_t st) {
     k_energy_members<<<dim3(nblocks, members), 256, 0, st>>>(e, n, partial);
     COUNT_LAUNCH(1);
 }
