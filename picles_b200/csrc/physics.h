@@ -57,6 +57,19 @@ namespace picles {
 inline int ph_host_specialised = 0;
 #endif
 
+/* the advance kernel a step launches (launch_advance, picles_kernels.cu; the specialised host build runs the same
+   copy): the TSIT5 template argument of k_advance, whose AUTOSW is solver == AutoTsit5.  1 Tsit5 and 2 DP5 on a
+   uniform kernel (their tableaus at compile time), 3 AutoTsit5: each takes propagation as on; 0 the generic one,
+   which also serves the reference's propagation = false switch.  nan_eest_rejects lives in the generic one only: the
+   specialised ones keep the code they were measured with. */
+inline int ph_advance_variant(const picles_params_t& P, bool per_node_M) {
+    if (!P.propagation || P.nan_eest_rejects) return 0;
+    if (P.solver == PICLES_SOLVER_AUTOTSIT5) return 3;
+    if (P.solver == PICLES_SOLVER_TSIT5) return 1;
+    if (P.solver == PICLES_SOLVER_DP5 && !per_node_M) return 2; /* -1.5 % on the bench06 settings */
+    return 0;
+}
+
 /* ---- tableaus (OrdinaryDiffEq Tsit5ConstantCache / DP5ConstantCache) ----- */
 /* a[s][j]: weight of k_j in the argument of stage s (s = 2..7, j = 1..s-1; row 7 = b);
    c[s-1]: time fraction of stage s; bt[j]: error weights (btilde). */
@@ -799,7 +812,7 @@ PM_HD bool integrate(const picles_params_t& P, const double wu0, const double wv
     const Tableau& T = nz ? tableau(PICLES_SOLVER_TSIT5) : (dz ? tableau(PICLES_SOLVER_DP5) : tableau(P.solver));
 #define PH_COEF_ON(c, can_be_zero) (nz || (dz && !(can_be_zero)) || (c) != 0.0)
     /* prop() in the attempt loop: the Tsit5 / DP5 instantiations are launched with propagation on only
-       (launch_advance; the host build selects them the same way), so they carry no test per stage; the
+       (ph_advance_variant), so they carry no test per stage; the
        monitor-carrying kernels have a second instantiation for it, TSIT5 == 3 */
 #define PH_PROP(cx_, cy_, ox_, oy_)                                                              \
     do {                                                                                         \
@@ -927,7 +940,7 @@ PM_HD bool integrate(const picles_params_t& P, const double wu0, const double wv
                 /* step_reject_controller!: dt /= min(1/qmin, q11/gamma), q11 = EEst^beta1 */
                 double q11 = (EEst == 0.0) ? 1.0 : pm_exp(sc.t1);
 #if defined(__CUDA_ARCH__)
-                /* the specialised copies (TSIT5 != 0) are launched only with the switch off (launch_advance2): their
+                /* the specialised copies (TSIT5 != 0) are launched only with the switch off (ph_advance_variant): their
                    code is what it was before the switch existed */
                 dt_next = dt / pm_reject_factor(TSIT5 == 0 ? P.nan_eest_rejects : 0, q11, qmin, gamma);
 #else

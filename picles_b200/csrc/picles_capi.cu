@@ -11,6 +11,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <utility>
 #include <vector>
 
 #include "../../include/picles_b200.h"
@@ -529,15 +530,22 @@ static int need_ready(picles_t* h, bool seeded) {
     return 0;
 }
 
+/* the wind level in the t1 slots is also the t level: the first step of a seeded or restored run reads it from both */
+static int t_level_from_t1(picles_t* h) {
+    const size_t bytes = (size_t)nodes(h) * 8;
+    CK(cudaMemcpyAsync(h->A.u_t, h->A.u_t1, bytes, cudaMemcpyDeviceToDevice, h->stream));
+    CK(cudaMemcpyAsync(h->A.v_t, h->A.v_t1, bytes, cudaMemcpyDeviceToDevice, h->stream));
+    return PICLES_OK;
+}
+
 /* SeedParticle from the wind already in the t1 slots (the first step's t level, see picles_step) */
 static int seed_from_t1(picles_t* h) {
     DeviceArrays& A = h->A;
-    int64_t n = nodes(h);
     CK(cudaMemsetAsync(h->d_counters, 0, sizeof(DeviceCounters), h->stream));
     launch_seed(A, h->P, A.u_t1, A.v_t1, h->d_counters, h->sms, h->stream);
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(A.u_t, A.u_t1, (size_t)n * 8, cudaMemcpyDeviceToDevice, h->stream));
-    CK(cudaMemcpyAsync(A.v_t, A.v_t1, (size_t)n * 8, cudaMemcpyDeviceToDevice, h->stream));
+    int rc = t_level_from_t1(h);
+    if (rc) return rc;
     CK(cudaMemcpyAsync(&h->h_counters->n_seed_off, &h->d_counters->n_seed_off, sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     h->n_seed_off = h->h_counters->n_seed_off;
@@ -591,21 +599,36 @@ int picles_set_wind_midlevels(picles_t* h, int n_mid, const double* u_mid, const
     return PICLES_OK;
 }
 
+/* host wind levels (null: not given) come as (u, v) pairs */
+static int check_wind_pairs(picles_t* h, const double* u_t, const double* v_t, const double* u_t1, const double* v_t1) {
+    if ((u_t == nullptr) != (v_t == nullptr) || (u_t1 == nullptr) != (v_t1 == nullptr))
+        return fail(h, PICLES_ERR_ARG, "wind components must be given in pairs");
+    return PICLES_OK;
+}
+
+/* the wind slots of the next step, of which the caller writes the t level (new_t) and the t+DT level (new_t1).  A new
+   t+DT level without a new t level makes the previous step's t+DT level this step's t level: the slots are swapped,
+   nothing is copied.  A written level is no longer the one picles_stage_wind_mesh sampled (wm_t1_valid). */
+static void next_wind_levels(picles_t* h, bool new_t, bool new_t1) {
+    DeviceArrays& A = h->A;
+    if (new_t || new_t1) h->wm_t1_valid = false;
+    if (!new_t && new_t1) {
+        std::swap(A.u_t, A.u_t1);
+        std::swap(A.v_t, A.v_t1);
+    }
+}
+
 int picles_upload_winds(picles_t* h, const double* u_t, const double* v_t, const double* u_t1, const double* v_t1) {
     int rc = need_ready(h, true);
     if (rc) return rc;
+    rc = check_wind_pairs(h, u_t, v_t, u_t1, v_t1);
+    if (rc) return rc;
     DeviceArrays& A = h->A;
     size_t bytes = (size_t)nodes(h) * 8;
-    if ((u_t == nullptr) != (v_t == nullptr) || (u_t1 == nullptr) != (v_t1 == nullptr))
-        return fail(h, PICLES_ERR_ARG, "wind components must be given in pairs");
-    if (u_t || u_t1) h->wm_t1_valid = false;
+    next_wind_levels(h, u_t, u_t1);
     if (u_t) {
         CK(cudaMemcpyAsync(A.u_t, u_t, bytes, cudaMemcpyHostToDevice, h->stream));
         CK(cudaMemcpyAsync(A.v_t, v_t, bytes, cudaMemcpyHostToDevice, h->stream));
-    } else if (u_t1) {
-        /* the previous step's t+DT level is this step's t level: swap, no copy */
-        double* tu = A.u_t; A.u_t = A.u_t1; A.u_t1 = tu;
-        double* tv = A.v_t; A.v_t = A.v_t1; A.v_t1 = tv;
     }
     if (u_t1) {
         CK(cudaMemcpyAsync(A.u_t1, u_t1, bytes, cudaMemcpyHostToDevice, h->stream));
@@ -630,39 +653,19 @@ static int keep_lag_level(picles_t* h) {
     return PICLES_OK;
 }
 
-int picles_step_advance(picles_t* h, double t, double dt_model) {
-    int rc = need_ready(h, true);
-    if (rc) return rc;
-    (void)t;
-    if (!(dt_model > 0)) return fail(h, PICLES_ERR_ARG, "dt_model must be positive");
-    CK(cudaMemsetAsync(h->d_counters, 0, sizeof(DeviceCounters), h->stream));
-    CK(cudaMemsetAsync(h->A.rowreach, 0, (size_t)record_rows(h) * 4, h->stream));
-    CK(cudaEventRecord(h->ev[0], h->stream));
-    launch_advance(h->A, h->P, dt_model, h->d_counters, h->sms, h->stream, 0, nodes(h), 0);
-    CK(cudaEventRecord(h->ev[1], h->stream));
-    CK(cudaGetLastError());
-    h->timing_valid = false;
-    return keep_lag_level(h);
-}
-
 /* ---- upload + advance, pipelined over row blocks -------------------------------------------
  * begin_advance: wind-level bookkeeping (same semantics as picles_upload_winds), counters and
- * per-row reach zeroed, start event.  advance_rows: the host winds of rows [r0, r1) are copied on
+ * per-row reach zeroed, start event.  advance_range: the host winds of each block of rows are copied on
  * the copy stream and the advance of those rows starts as soon as they have landed, so block c
  * integrates while block c+1 is still in flight. */
 static int begin_advance(picles_t* h, double dt_model, const double* u_t, const double* v_t, const double* u_t1,
                          const double* v_t1) {
-    DeviceArrays& A = h->A;
-    if ((u_t == nullptr) != (v_t == nullptr) || (u_t1 == nullptr) != (v_t1 == nullptr))
-        return fail(h, PICLES_ERR_ARG, "wind components must be given in pairs");
+    int rc = check_wind_pairs(h, u_t, v_t, u_t1, v_t1);
+    if (rc) return rc;
     if (!(dt_model > 0)) return fail(h, PICLES_ERR_ARG, "dt_model must be positive");
-    if (u_t || u_t1) h->wm_t1_valid = false;
-    if (!u_t && u_t1) { /* the previous step's t+DT level is this step's t level: swap, no copy */
-        double* tu = A.u_t; A.u_t = A.u_t1; A.u_t1 = tu;
-        double* tv = A.v_t; A.v_t = A.v_t1; A.v_t1 = tv;
-    }
+    next_wind_levels(h, u_t, u_t1);
     CK(cudaMemsetAsync(h->d_counters, 0, sizeof(DeviceCounters), h->stream));
-    CK(cudaMemsetAsync(A.rowreach, 0, (size_t)record_rows(h) * 4, h->stream));
+    CK(cudaMemsetAsync(h->A.rowreach, 0, (size_t)record_rows(h) * 4, h->stream));
     if (u_t || u_t1) {
         /* the copy stream may only overwrite the wind planes once the compute stream is past
            every earlier kernel that read them */
@@ -692,52 +695,23 @@ static int upload_rows(picles_t* h, const double* u_t, const double* v_t, const 
     CK(cudaStreamWaitEvent(consumer, landed, 0));
     return PICLES_OK;
 }
-static int advance_rows(picles_t* h, double dt_model, const double* u_t, const double* v_t, const double* u_t1,
-                        const double* v_t1, int r0, int r1, cudaEvent_t landed, int slot) {
-    DeviceArrays& A = h->A;
-    if (r0 >= r1) return PICLES_OK;
-    const int64_t off = (int64_t)r0 * A.Nx;
-    const size_t bytes = (size_t)(r1 - r0) * A.Nx * 8;
-    if (u_t) {
-        CK(cudaMemcpyAsync(A.u_t + off, u_t + off, bytes, cudaMemcpyHostToDevice, h->copy_stream));
-        CK(cudaMemcpyAsync(A.v_t + off, v_t + off, bytes, cudaMemcpyHostToDevice, h->copy_stream));
-    }
-    if (u_t1) {
-        CK(cudaMemcpyAsync(A.u_t1 + off, u_t1 + off, bytes, cudaMemcpyHostToDevice, h->copy_stream));
-        CK(cudaMemcpyAsync(A.v_t1 + off, v_t1 + off, bytes, cudaMemcpyHostToDevice, h->copy_stream));
-    }
-    if (u_t || u_t1) {
-        CK(cudaEventRecord(landed, h->copy_stream));
-        CK(cudaStreamWaitEvent(h->stream, landed, 0));
-    }
-    launch_advance(A, h->P, dt_model, h->d_counters, h->sms, h->stream, off, off + (int64_t)(r1 - r0) * A.Nx, slot);
-    return PICLES_OK;
-}
-/* rows [r0, r1) in up to PIPE_CHUNKS blocks (one block when nothing is uploaded or the range is small) */
+/* rows [r0, r1), block c on work queue c.  Graded blocks when host winds are uploaded and the range has at least
+   PIPE_MIN_NODES nodes, one block otherwise: 64 rows first, each next block three times the one before (an upload
+   takes about a third of the advance of the same rows, so it still hides), the last takes the rest.  Only the first
+   block's upload is exposed: 0.08 ms instead of the 0.6 ms of eight equal blocks at 4096^2 (end to end 16.39 -> 15.76
+   ms per step, profiles/README.md). */
 static int advance_range(picles_t* h, double dt_model, const double* u_t, const double* v_t, const double* u_t1,
                          const double* v_t1, int r0, int r1) {
-    const int64_t n = (int64_t)(r1 - r0) * h->A.Nx;
-    const int nch = ((u_t || u_t1) && n >= PIPE_MIN_NODES) ? PIPE_CHUNKS : 1;
-    /* graded blocks: 64 rows first, each next block three times the one before (an upload takes about a third of the
-       advance of the same rows, so it still hides), the last takes the rest.  Only the first block's upload is
-       exposed: 0.08 ms instead of the 0.6 ms of eight equal blocks at 4096^2 (end to end 16.39 -> 15.76 ms per step,
-       profiles/README.md).  PICLES_PIPE_FIRST_ROWS=k overrides the first block; 0 = equal blocks. */
-    static const int first_rows = [] { const char* e = getenv("PICLES_PIPE_FIRST_ROWS"); return e ? atoi(e) : 64; }();
-    if (nch > 1 && first_rows > 0) {
-        int a = r0, len = first_rows;
-        for (int c = 0; c < PIPE_CHUNKS && a < r1; c++) {
-            const int b = (c == PIPE_CHUNKS - 1 || a + len >= r1) ? r1 : a + len;
-            int rc = advance_rows(h, dt_model, u_t, v_t, u_t1, v_t1, a, b, h->pev[c], c);
-            if (rc) return rc;
-            a = b; len *= 3;
-        }
-        return PICLES_OK;
-    }
-    const int rows = (r1 - r0 + nch - 1) / nch;
-    for (int c = 0; c < nch; c++) {
-        const int a = r0 + c * rows, b = (a + rows < r1) ? a + rows : r1;
-        int rc = advance_rows(h, dt_model, u_t, v_t, u_t1, v_t1, a, b, h->pev[c], c);
+    const DeviceArrays& A = h->A;
+    const bool graded = (u_t || u_t1) && (int64_t)(r1 - r0) * A.Nx >= PIPE_MIN_NODES;
+    int a = r0, len = 64;
+    for (int c = 0; c < PIPE_CHUNKS && a < r1; c++) {
+        const int b = (!graded || c == PIPE_CHUNKS - 1 || a + len >= r1) ? r1 : a + len;
+        int rc = upload_rows(h, u_t, v_t, u_t1, v_t1, a, b, h->pev[c], h->stream);
         if (rc) return rc;
+        const int64_t l_end = (int64_t)b * A.Nx;
+        launch_advance(A, h->P, dt_model, h->d_counters, h->sms, h->stream, (int64_t)a * A.Nx, l_end, l_end, l_end, c);
+        a = b; len *= 3;
     }
     return PICLES_OK;
 }
@@ -751,6 +725,13 @@ static int upload_and_advance(picles_t* h, double dt_model, const double* u_t, c
     CK(cudaEventRecord(h->ev[1], h->stream));
     CK(cudaGetLastError());
     return keep_lag_level(h);
+}
+
+int picles_step_advance(picles_t* h, double t, double dt_model) {
+    int rc = need_ready(h, true);
+    if (rc) return rc;
+    (void)t;
+    return upload_and_advance(h, dt_model, nullptr, nullptr, nullptr, nullptr);
 }
 
 int picles_get_reach(picles_t* h, int32_t* reach) {
@@ -1319,8 +1300,8 @@ int picles_checkpoint_load(picles_t* h, const void* blob, int64_t nbytes) {
     /* no deposit records are carried over: every step rewrites them before they are read */
     const int64_t ne = (int64_t)A.rp * (A.ny + 2 * A.halo);
     launch_fill_i32(A.cell, ne, -1, h->sms, h->stream);
-    CK(cudaMemcpyAsync(A.u_t, A.u_t1, (size_t)n * 8, cudaMemcpyDeviceToDevice, h->stream));
-    CK(cudaMemcpyAsync(A.v_t, A.v_t1, (size_t)n * 8, cudaMemcpyDeviceToDevice, h->stream));
+    rc = t_level_from_t1(h);
+    if (rc) return rc;
     CK(cudaStreamSynchronize(h->stream));
     CK(cudaGetLastError());
     A.u_lag = with_lag ? h->lag_u : nullptr;
@@ -1469,8 +1450,8 @@ int picles_step_strip(picles_t* h, double t, double dt_model, const double* u_t,
         if (rc) return rc;
         rc = upload_rows(h, u_t, v_t, u_t1, v_t1, A.ny - hb, A.ny, h->pev[PIPE_CHUNKS + 1], h->comm_stream);
         if (rc) return rc;
-        launch_advance2(A, h->P, dt_model, h->d_counters, h->sms, h->comm_stream, 0, (int64_t)hb * A.Nx,
-                        (int64_t)(A.ny - hb) * A.Nx, (int64_t)A.ny * A.Nx, ADV_SLOT_BOUNDARY);
+        launch_advance(A, h->P, dt_model, h->d_counters, h->sms, h->comm_stream, 0, (int64_t)hb * A.Nx,
+                       (int64_t)(A.ny - hb) * A.Nx, (int64_t)A.ny * A.Nx, ADV_SLOT_BOUNDARY);
         CK(cudaGetLastError());
         if (u_t || u_t1) { /* whole-plane readers on the compute stream (the lag-level copy, the remesh) see the boundary rows too */
             CK(cudaStreamWaitEvent(h->stream, h->pev[PIPE_CHUNKS], 0));
@@ -1650,12 +1631,10 @@ int picles_stage_wind_mesh(picles_t* h, double t, double dt_model, int n_mid) {
     DeviceArrays& A = h->A;
     rc = ensure_mid_planes(h, n_mid);
     if (rc) return rc;
-    if (h->wm_t1_valid && h->wm_t1_time == t) { /* the previous step's t+dt level is this step's t level */
-        double* tu = A.u_t; A.u_t = A.u_t1; A.u_t1 = tu;
-        double* tv = A.v_t; A.v_t = A.v_t1; A.v_t1 = tv;
-    } else {
-        wind_sample(h, t, A.u_t, A.v_t);
-    }
+    /* false: the previous step's t+dt level is this step's t level */
+    const bool new_t = !(h->wm_t1_valid && h->wm_t1_time == t);
+    next_wind_levels(h, new_t, true);
+    if (new_t) wind_sample(h, t, A.u_t, A.v_t);
     const double t1 = t + dt_model;
     wind_sample(h, t1, A.u_t1, A.v_t1);
     for (int k = 1; k <= n_mid; k++)

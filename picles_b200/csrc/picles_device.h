@@ -106,9 +106,7 @@ struct DeviceCounters {
 void launch_seed(const DeviceArrays& A, const picles_params_t& P, const double* u0, const double* v0, DeviceCounters* dc,
                  int sms, cudaStream_t st);
 void launch_advance(const DeviceArrays& A, const picles_params_t& P, double DT, DeviceCounters* dc, int sms,
-                    cudaStream_t st, int64_t l_begin, int64_t l_end, int slot);
-void launch_advance2(const DeviceArrays& A, const picles_params_t& P, double DT, DeviceCounters* dc, int sms,
-                     cudaStream_t st, int64_t l_begin, int64_t l_end, int64_t l2_begin, int64_t l2_end, int slot);
+                    cudaStream_t st, int64_t l_begin, int64_t l_end, int64_t l2_begin, int64_t l2_end, int slot);
 /* *dst = *src + 1 on the stream: the word the strips all-reduce (1 + reach, so that 0 reads as "not set") */
 void launch_reach_word(const int32_t* src, int32_t* dst, cudaStream_t st);
 /* kernels launched by this library since it was loaded (every launch_* call counts its kernels) */

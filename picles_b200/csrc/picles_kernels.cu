@@ -944,110 +944,77 @@ void launch_seed(const DeviceArrays& A, const picles_params_t& P, const double* 
     COUNT_LAUNCH(1);
 }
 
-/* launch_advance2 for an ensemble: the same choice of instantiation, each in its ensemble form */
-static void launch_advance_members(const DeviceArrays& A, const picles_params_t& P, double DT, DeviceCounters* dc, int sms,
-                                   cudaStream_t st, int64_t l_begin, int64_t l_end, int64_t l2_begin, int64_t l2_end,
-                                   int slot, int g, bool pn) {
-    const int64_t count = (l_end - l_begin) + (l2_end - l2_begin);
-    const bool spec = !P.nan_eest_rejects;
-#define ADV_ARGS A, P, DT, dc, l_begin, l_end, l2_begin, l2_end, slot
-    if (P.solver == PICLES_SOLVER_AUTOTSIT5) {
-        const int gr = grid_for(count, ADV_THREADS, sms, 1);
-        if (pn) {
-            if (P.propagation && spec) k_advance<true, true, 3, true><<<g, ADV_THREADS, 0, st>>>(ADV_ARGS);
-            else k_advance<true, true, 0, true><<<g, ADV_THREADS, 0, st>>>(ADV_ARGS);
-            k_advance_resume<true, true><<<gr, ADV_THREADS, 0, st>>>(A, P, DT, dc, l_begin, l_end);
-        } else {
-            if (P.propagation && spec) k_advance<false, true, 3, true><<<g, ADV_THREADS, 0, st>>>(ADV_ARGS);
-            else k_advance<false, true, 0, true><<<g, ADV_THREADS, 0, st>>>(ADV_ARGS);
-            k_advance_resume<false, true><<<gr, ADV_THREADS, 0, st>>>(A, P, DT, dc, l_begin, l_end);
-        }
-        COUNT_LAUNCH(2);
-    } else {
-        const bool ts5 = (P.solver == PICLES_SOLVER_TSIT5) && P.propagation && spec;
-        if (pn && ts5) k_advance<true, false, 1, true><<<g, ADV_THREADS, 0, st>>>(ADV_ARGS);
-        else if (pn) k_advance<true, false, 0, true><<<g, ADV_THREADS, 0, st>>>(ADV_ARGS);
-        else if (ts5) k_advance<false, false, 1, true><<<g, ADV_THREADS, 0, st>>>(ADV_ARGS);
-        else if (P.solver == PICLES_SOLVER_DP5 && P.propagation && spec) k_advance<false, false, 2, true><<<g, ADV_THREADS, 0, st>>>(ADV_ARGS);
-        else k_advance<false, false, 0, true><<<g, ADV_THREADS, 0, st>>>(ADV_ARGS);
+/* k_advance<PER_NODE_M, AUTOSW, TSIT5, ENS> over the particles of both ranges; under AutoTsit5, then the Rosenbrock23
+   finish of the particles it parked (k_advance_resume) */
+template <bool PER_NODE_M, bool AUTOSW, int TSIT5, bool ENS>
+static void advance_kernels(const DeviceArrays& A, const picles_params_t& P, double DT, DeviceCounters* dc, int sms,
+                            cudaStream_t st, int64_t l_begin, int64_t l_end, int64_t l2_begin, int64_t l2_end, int slot,
+                            int64_t count) {
+    k_advance<PER_NODE_M, AUTOSW, TSIT5, ENS><<<grid_for(count, ADV_THREADS, sms, ADV_MIN_BLOCKS), ADV_THREADS, 0, st>>>(
+        A, P, DT, dc, l_begin, l_end, l2_begin, l2_end, slot);
+    COUNT_LAUNCH(1);
+    if constexpr (AUTOSW) {
+        k_advance_resume<PER_NODE_M, ENS><<<grid_for(count, ADV_THREADS, sms, 1), ADV_THREADS, 0, st>>>(A, P, DT, dc, l_begin, l_end);
         COUNT_LAUNCH(1);
     }
-#undef ADV_ARGS
+}
+
+/* the instantiation ph_advance_variant picks (physics.h), in its single-model or ensemble form: one branch per
+   instantiation the library has, so nothing else is compiled */
+template <bool ENS>
+static void launch_advance_as(const DeviceArrays& A, const picles_params_t& P, double DT, DeviceCounters* dc, int sms,
+                              cudaStream_t st, int64_t l_begin, int64_t l_end, int64_t l2_begin, int64_t l2_end, int slot,
+                              int64_t count) {
+#define ADV(PER_NODE_M, AUTOSW, TSIT5) \
+    advance_kernels<PER_NODE_M, AUTOSW, TSIT5, ENS>(A, P, DT, dc, sms, st, l_begin, l_end, l2_begin, l2_end, slot, count)
+    const bool pn = (A.M[0] != nullptr);
+    const int v = ph_advance_variant(P, pn);
+    if (P.solver == PICLES_SOLVER_AUTOTSIT5) {
+        if (pn && v == 3) ADV(true, true, 3);
+        else if (pn) ADV(true, true, 0);
+        else if (v == 3) ADV(false, true, 3);
+        else ADV(false, true, 0);
+    } else if (pn && v == 1) ADV(true, false, 1);
+    else if (pn) ADV(true, false, 0);
+    else if (v == 1) ADV(false, false, 1);
+    else if (v == 2) ADV(false, false, 2);
+    else ADV(false, false, 0);
+#undef ADV
 }
 
 /* particles [l_begin, l_end) and then [l2_begin, l2_end) of the strip (the whole strip: 0, Nx*ny and an empty
    second range); slot: the work queue of this launch (DeviceCounters::next_chunk, zeroed with the counters at the
    start of the step) */
-void launch_advance2(const DeviceArrays& A, const picles_params_t& P, double DT, DeviceCounters* dc, int sms,
-                     cudaStream_t st, int64_t l_begin, int64_t l_end, int64_t l2_begin, int64_t l2_end, int slot) {
+void launch_advance(const DeviceArrays& A, const picles_params_t& P, double DT, DeviceCounters* dc, int sms,
+                    cudaStream_t st, int64_t l_begin, int64_t l_end, int64_t l2_begin, int64_t l2_end, int slot) {
     if (l2_end < l2_begin) l2_end = l2_begin;
     if (l_end < l_begin) l_end = l_begin;
     const int64_t count = (l_end - l_begin) + (l2_end - l2_begin);
     if (count <= 0) return;
-    int g = grid_for(count, ADV_THREADS, sms, ADV_MIN_BLOCKS);
-    bool pn = (A.M[0] != nullptr);
-    if (A.members > 1) {
-        launch_advance_members(A, P, DT, dc, sms, st, l_begin, l_end, l2_begin, l2_end, slot, g, pn);
-        return;
-    }
-    /* picles_params_t::nan_eest_rejects (a NaN error estimate rejected by 1/qmin instead of ending the integrator) lives
-       in the generic instantiations only: the specialised ones keep the code they were measured with */
-    const bool spec = !P.nan_eest_rejects;
-#define ADV_ARGS A, P, DT, dc, l_begin, l_end, l2_begin, l2_end, slot
-    /* AutoTsit5 runs the instantiation that carries the stiffness monitor and the Rosenbrock23 branch */
-    if (P.solver == PICLES_SOLVER_AUTOTSIT5) {
-        const int gr = grid_for(count, ADV_THREADS, sms, 1);
-        /* (third template argument 3: propagation on, known at compile time, as in the Tsit5 / DP5 instantiations) */
-        if (pn) {
-            if (P.propagation && spec) k_advance<true, true, 3><<<g, ADV_THREADS, 0, st>>>(ADV_ARGS);
-            else k_advance<true, true><<<g, ADV_THREADS, 0, st>>>(ADV_ARGS);
-            k_advance_resume<true><<<gr, ADV_THREADS, 0, st>>>(A, P, DT, dc, l_begin, l_end);
-        } else {
-            if (P.propagation && spec) k_advance<false, true, 3><<<g, ADV_THREADS, 0, st>>>(ADV_ARGS);
-            else k_advance<false, true><<<g, ADV_THREADS, 0, st>>>(ADV_ARGS);
-            k_advance_resume<false><<<gr, ADV_THREADS, 0, st>>>(A, P, DT, dc, l_begin, l_end);
-        }
-        COUNT_LAUNCH(2);
-    } else {
-        /* Tsit5 has its own instantiation (compile-time tableau without zero coefficients) */
-        /* (the specialised instantiations take propagation as given: a run without it — the reference's
-           propagation = false switch — is served by the generic one) */
-        const bool ts5 = (P.solver == PICLES_SOLVER_TSIT5) && P.propagation && spec;
-        if (pn && ts5) k_advance<true, false, true><<<g, ADV_THREADS, 0, st>>>(ADV_ARGS);
-        else if (pn) k_advance<true, false><<<g, ADV_THREADS, 0, st>>>(ADV_ARGS);
-        else if (ts5) k_advance<false, false, true><<<g, ADV_THREADS, 0, st>>>(ADV_ARGS);
-        /* ... and so has DP5 on a uniform kernel (the bench06 settings): -1.5 % */
-        else if (P.solver == PICLES_SOLVER_DP5 && P.propagation && spec) k_advance<false, false, 2><<<g, ADV_THREADS, 0, st>>>(ADV_ARGS);
-        else k_advance<false, false><<<g, ADV_THREADS, 0, st>>>(ADV_ARGS);
-        COUNT_LAUNCH(1);
-    }
-#undef ADV_ARGS
-}
-void launch_advance(const DeviceArrays& A, const picles_params_t& P, double DT, DeviceCounters* dc, int sms,
-                    cudaStream_t st, int64_t l_begin, int64_t l_end, int slot) {
-    launch_advance2(A, P, DT, dc, sms, st, l_begin, l_end, l_end, l_end, slot);
+    if (A.members > 1) launch_advance_as<true>(A, P, DT, dc, sms, st, l_begin, l_end, l2_begin, l2_end, slot, count);
+    else launch_advance_as<false>(A, P, DT, dc, sms, st, l_begin, l_end, l2_begin, l2_end, slot, count);
 }
 
 int project_remesh_smem_bytes() { return (int)sizeof(PRTile) + 128; }
-cudaError_t project_remesh_configure() {
-    const int b = project_remesh_smem_bytes();
-    cudaError_t e = cudaFuncSetAttribute(k_project_remesh<PR_HY_NARROW>, cudaFuncAttributeMaxDynamicSharedMemorySize, b);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_project_remesh<PR_HY_WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, b);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_project_remesh<PR_HY_NARROW, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, b);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_project_remesh<PR_HY_WIDE, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, b);
-    return e;
-}
 /* wide: cut the 72 x 20 box as 12 target rows + 4 halo rows (previous step's reach was 3-4)
    instead of 16 + 2; a wrong guess only sends tiles through the generic gather */
+static auto project_remesh_kernel(bool wide, bool ens) {
+    return ens ? (wide ? k_project_remesh<PR_HY_WIDE, true> : k_project_remesh<PR_HY_NARROW, true>)
+               : (wide ? k_project_remesh<PR_HY_WIDE, false> : k_project_remesh<PR_HY_NARROW, false>);
+}
+cudaError_t project_remesh_configure() {
+    cudaError_t e = cudaSuccess;
+    for (int k = 0; k < 4 && e == cudaSuccess; k++)
+        e = cudaFuncSetAttribute(project_remesh_kernel(k & 1, k & 2), cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 project_remesh_smem_bytes());
+    return e;
+}
 void launch_project_remesh(const ProjectMaps& maps, const DeviceArrays& A, const picles_params_t& P, double DT,
                            int n_classes, int accumulate, int wide, DeviceCounters* dc, cudaStream_t st) {
     const int TY = PR_BH - 2 * (wide ? PR_HY_WIDE : PR_HY_NARROW);
     dim3 grid((A.Nx + PR_TX - 1) / PR_TX, (A.ny + TY - 1) / TY, A.members);
-    if (A.members > 1) {
-        if (wide) k_project_remesh<PR_HY_WIDE, true><<<grid, PR_THREADS, project_remesh_smem_bytes(), st>>>(maps, A, P, DT, n_classes, accumulate, dc);
-        else k_project_remesh<PR_HY_NARROW, true><<<grid, PR_THREADS, project_remesh_smem_bytes(), st>>>(maps, A, P, DT, n_classes, accumulate, dc);
-    } else if (wide) k_project_remesh<PR_HY_WIDE><<<grid, PR_THREADS, project_remesh_smem_bytes(), st>>>(maps, A, P, DT, n_classes, accumulate, dc);
-    else k_project_remesh<PR_HY_NARROW><<<grid, PR_THREADS, project_remesh_smem_bytes(), st>>>(maps, A, P, DT, n_classes, accumulate, dc);
+    project_remesh_kernel(wide, A.members > 1)<<<grid, PR_THREADS, project_remesh_smem_bytes(), st>>>(
+        maps, A, P, DT, n_classes, accumulate, dc);
     COUNT_LAUNCH(1);
 }
 

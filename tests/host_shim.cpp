@@ -61,19 +61,9 @@ static void tally_add(Tally& a, const Tally& b) {
 
 extern "C" {
 
-/* the third template argument of the k_advance instantiation launch_advance2 launches (picles_kernels.cu): 1 Tsit5,
-   2 DP5 on a uniform kernel, 3 AutoTsit5, each with propagation on and nan_eest_rejects off; 0 the generic ones.  The
-   specialised host build runs the same copy for 1, 2 and 3.  For 0 it runs advance_particle<true, 0> whatever the
-   solver, where the device's generic Tsit5 / DP5 kernels run advance_particle<false, 0>: on the host the monitor is
-   gated on the solver at run time (physics.h integrate), so both compute the same. */
-int shim_advance_template(const picles_params_t* P, int per_node_M) {
-    const bool spec = !P->nan_eest_rejects;
-    if (!P->propagation || !spec) return 0;
-    if (P->solver == PICLES_SOLVER_AUTOTSIT5) return 3;
-    if (P->solver == PICLES_SOLVER_TSIT5) return 1;
-    if (P->solver == PICLES_SOLVER_DP5 && !per_node_M) return 2;
-    return 0;
-}
+/* the third template argument of the k_advance instantiation the library launches (physics.h: ph_advance_variant),
+   which the specialised host build runs the same copy of, for the tests to hold to their mirror */
+int shim_advance_template(const picles_params_t* P, int per_node_M) { return ph_advance_variant(*P, per_node_M); }
 
 Shim* shim_create(int Nx, int Ny, int bx, int by, int nstrips, int halo, const uint8_t* mask, const double* M,
                   const double* M_const, const double* pc, const picles_params_t* P) {
@@ -188,8 +178,10 @@ static void shim_advance_all(Shim* h, double DT, const double* u_t, const double
             /* as k_advance: a particle seeded off under B-1 as run reads the level kept from the first step */
             double wu1 = u_t1[off + l], wv1 = v_t1[off + l];
             if (!s.ulag.empty() && !(p.flags & PICLES_PF_ON)) { wu1 = s.ulag[l]; wv1 = s.vlag[l]; }
-            /* as launch_advance2 picks the kernel */
-            const int tsit5 = ph_host_specialised ? shim_advance_template(&h->P, h->perM) : 0;
+            /* as launch_advance picks the kernel.  For 0 the host runs advance_particle<true, 0> whatever the solver,
+               where the device's generic Tsit5 / DP5 kernels run advance_particle<false, 0>: on the host the monitor
+               is gated on the solver at run time (physics.h integrate), so both compute the same. */
+            const int tsit5 = ph_host_specialised ? ph_advance_variant(h->P, h->perM) : 0;
             const bool pending = (tsit5 == 1)
                 ? advance_particle<false, 1>(h->P, p, s.mask[l], DT, u_t[off + l], v_t[off + l], wu1,
                                              wv1, h->n_mid, um, vm, M, pc, r, c, K, attempts)

@@ -1,4 +1,4 @@
-"""CPU tests of the advance-kernel cases (tests/advance_cases.py): the selection mirror against the launch sites of
+"""CPU tests of the advance-kernel cases (tests/advance_cases.py): the selection mirror against the launcher of
 picles_kernels.cu, proof that the cases launch all 22 advance kernels and reach every device-only path they claim,
 the host build of the device header against the oracle on every case, and the oracle's right-hand side against
 exact arithmetic at the premise edges the cases push the kernels to."""
@@ -16,12 +16,12 @@ import advance_cases as AC
 from common import HostShim, PiclesParams, ROOT, compare_models, default_params, make_oracle, shim_lib
 
 KERNELS_CU = os.path.join(ROOT, "picles_b200", "csrc", "picles_kernels.cu")
-LAUNCHERS = ("launch_advance_members", "launch_advance2")
+LAUNCHERS = ("advance_kernels", "launch_advance_as", "launch_advance")
 
 
 def _function_text(src, name):
-    """the definition of `name` in src, from its return type to its closing brace"""
-    m = re.search(r"^(?:static\s+)?void\s+" + name + r"\(", src, re.M)
+    """the definition of `name` in src, from its template head or return type to its closing brace"""
+    m = re.search(r"^(?:template\s*<[^>]*>\s*)?(?:static\s+)?void\s+" + name + r"\(", src, re.M)
     assert m, name
     i = src.index("{", m.end())
     depth = 0
@@ -41,39 +41,53 @@ def _template_head(src, kernel):
 
 @pytest.fixture(scope="module")
 def launch_selection(tmp_path_factory):
-    """launch_advance_members and launch_advance2 as they stand in picles_kernels.cu, compiled for the host with every
-    kernel launch replaced by a call that records its template arguments (default arguments filled in by the
-    compiler from the kernels' own template heads) and the launch counter kept as the library keeps it"""
+    """launch_advance and the templates behind it as they stand in picles_kernels.cu, compiled for the host with
+    physics.h (ph_advance_variant) and every kernel launch replaced by a call that records its template arguments
+    (default arguments filled in by the compiler from the kernels' own template heads), with the launch counter kept
+    as the library keeps it.  Each recorder instantiation registers itself when the library is loaded, so the
+    registry lists every kernel the launcher can launch, whether or not some call reaches it."""
     src = open(KERNELS_CU).read()
     bodies = [_function_text(src, f) for f in LAUNCHERS]
     launch = re.compile(r"\b(k_advance(?:_resume)?)<([^<>]*)><<<[^>]*>>>\([^;]*\);")
-    n_sites = sum(len(launch.findall(b)) for b in bodies)
+    assert any(launch.search(b) for b in bodies)
     bodies = [launch.sub(r"\1_rec<\2>();", b) for b in bodies]
+    body_text = "\n".join(bodies)
     code = f"""
 #include <cstdint>
-#include "picles_b200.h"
+#include "physics.h"
+using namespace picles;
 typedef void* cudaStream_t;
 struct DeviceCounters;
 struct DeviceArrays {{ int members; const double* M[4]; }};
 #define ADV_THREADS 128
 #define ADV_MIN_BLOCKS 1
-static int rec_n = 0, rec_launches = 0;
-static int rec_k[16][5];
+#define REG_MAX 64
+static int n_reg = 0, reg[REG_MAX][5]; /* every recorder instantiation: kind, PER_NODE_M, AUTOSW, TSIT5, ENS */
+static int rec_n = 0, rec[16], rec_launches = 0;
 #define COUNT_LAUNCH(n) (rec_launches += (n))
 static int grid_for(int64_t, int, int, int) {{ return 1; }}
+static int add_reg(int kind, int pn, int autosw, int tsit5, int ens) {{
+    if (n_reg < REG_MAX) {{ int* r = reg[n_reg]; r[0] = kind; r[1] = pn; r[2] = autosw; r[3] = tsit5; r[4] = ens; }}
+    return n_reg++;
+}}
+template <bool PN, bool AUTOSW, int TSIT5, bool ENS> int k_advance_id = add_reg(0, PN, AUTOSW, TSIT5, ENS);
+template <bool PN, bool ENS> int k_advance_resume_id = add_reg(1, PN, 0, 0, ENS);
 template <{_template_head(src, "k_advance")}> void k_advance_rec() {{
-    int* r = rec_k[rec_n++]; r[0] = 0; r[1] = PER_NODE_M; r[2] = AUTOSW; r[3] = TSIT5; r[4] = ENS; }}
+    rec[rec_n++] = k_advance_id<PER_NODE_M, AUTOSW, TSIT5, ENS>; }}
 template <{_template_head(src, "k_advance_resume")}> void k_advance_resume_rec() {{
-    int* r = rec_k[rec_n++]; r[0] = 1; r[1] = PER_NODE_M; r[2] = 0; r[3] = 0; r[4] = ENS; }}
-{bodies[0]}
-{bodies[1]}
+    rec[rec_n++] = k_advance_resume_id<PER_NODE_M, ENS>; }}
+{body_text}
+extern "C" int registered(int* out) {{
+    for (int i = 0; i < n_reg && i < REG_MAX; i++) for (int c = 0; c < 5; c++) out[5 * i + c] = reg[i][c];
+    return n_reg;
+}}
 extern "C" int select_kernels(const picles_params_t* P, int per_node_M, int members, int* out, int* launches) {{
     static const double plane = 0.0;
     DeviceArrays A; A.members = members;
     for (int k = 0; k < 4; k++) A.M[k] = per_node_M ? &plane : nullptr;
     rec_n = 0; rec_launches = 0;
-    launch_advance2(A, *P, 600.0, nullptr, 148, nullptr, 0, 64, 64, 64, 0);
-    for (int i = 0; i < rec_n; i++) for (int c = 0; c < 5; c++) out[5 * i + c] = rec_k[i][c];
+    launch_advance(A, *P, 600.0, nullptr, 148, nullptr, 0, 64, 64, 64, 0);
+    for (int i = 0; i < rec_n; i++) for (int c = 0; c < 5; c++) out[5 * i + c] = reg[rec[i]][c];
     *launches = rec_launches;
     return rec_n;
 }}
@@ -81,39 +95,49 @@ extern "C" int select_kernels(const picles_params_t* P, int per_node_M, int memb
     d = tmp_path_factory.mktemp("launch_selection")
     cpp, so = d / "sel.cpp", d / "libsel.so"
     cpp.write_text(code)
-    r = subprocess.run(["g++", "-std=c++17", "-O0", "-shared", "-fPIC", "-I", os.path.join(ROOT, "include"), "-o",
-                        str(so), str(cpp)], capture_output=True, text=True)
+    r = subprocess.run(["g++", "-std=c++17", "-O0", "-shared", "-fPIC", "-I", os.path.join(ROOT, "picles_b200", "csrc"),
+                        "-o", str(so), str(cpp)], capture_output=True, text=True)
     assert r.returncode == 0, r.stderr
     lib = C.CDLL(str(so))
     lib.select_kernels.restype = C.c_int
     lib.select_kernels.argtypes = [C.POINTER(PiclesParams), C.c_int, C.c_int, C.c_void_p, C.c_void_p]
+    lib.registered.restype = C.c_int
+    lib.registered.argtypes = [C.c_void_p]
+
+    def kernels(rows):
+        ks = set()
+        for row in rows:
+            if row[0] == 0:
+                ks.add(("k_advance", bool(row[1]), bool(row[2]), int(row[3]), bool(row[4])))
+            else:
+                ks.add(("k_advance_resume", bool(row[1]), bool(row[4])))
+        assert len(ks) == len(rows)
+        return ks
 
     def select(P, pn, members):
         out = np.zeros((16, 5), np.int32)
         nl = np.zeros(1, np.int32)
         n = lib.select_kernels(C.byref(P), int(pn), int(members), out.ctypes.data, nl.ctypes.data)
-        ks = set()
-        for row in out[:n]:
-            if row[0] == 0:
-                ks.add(("k_advance", bool(row[1]), bool(row[2]), int(row[3]), bool(row[4])))
-            else:
-                ks.add(("k_advance_resume", bool(row[1]), bool(row[4])))
-        assert len(ks) == n
-        return ks, int(nl[0])
-    select.n_sites = n_sites
+        return kernels(out[:n]), int(nl[0])
+
+    out = np.zeros((64, 5), np.int32)
+    n = lib.registered(out.ctypes.data)
+    assert n <= len(out), n
+    select.instantiated = kernels(out[:n])
     return select
 
 
 def _combinations():
     for solver, prop, nan_eest, pn, E in itertools.product(("Tsit5", "DP5", "AutoTsit5"), (True, False), (False, True),
-                                                          (False, True), (1, 3)):
+                                                          (False, True), (1, 2, 3)):
         yield default_params(solver=solver, propagation=prop, nan_eest_rejects=nan_eest), pn, E
 
 
-def test_selection_mirror_equals_the_launch_sites(launch_selection):
+def test_selection_mirror_equals_the_launcher(launch_selection):
     """for every solver x propagation x nan_eest_rejects x per-node kernel x (E = 1, E > 1), the kernels the source
-    launches are the mirror's, and the library counts one launch per kernel; over all of them, the 22 kernels"""
-    assert launch_selection.n_sites == len(AC.ALL_KERNELS)
+    launches are the mirror's, and the library counts one launch per kernel; over all of them, the 22 kernels, and the
+    launcher can launch no other"""
+    assert launch_selection.instantiated == AC.ALL_KERNELS
     image = set()
     for P, pn, E in _combinations():
         got, launches = launch_selection(P, pn, E)
@@ -125,7 +149,7 @@ def test_selection_mirror_equals_the_launch_sites(launch_selection):
 
 
 def test_host_build_selects_as_the_device():
-    """the specialised host build runs the copy of the instantiation launch_advance2 would launch"""
+    """the specialised host build runs the copy of the instantiation launch_advance would launch"""
     lib = shim_lib()
     for P, pn, E in _combinations():
         if E == 1:
