@@ -294,7 +294,14 @@ struct OpsSafe {
     static PM_HDM double exp_(double x, unsigned*) { return pm_exp(x); }
     static PM_HDM double pow_(double x, double y, unsigned*) { return pm_pow_safe(x, y); }
     static PM_HDM double log_(double x, unsigned*) { return pm_log_safe(x); }
+    static PM_HDM double log_pos(double x, unsigned*) { return pm_log_safe(x); }
     static PM_HDM double log10_(double x, unsigned*) { return pm_log10_safe(x); }
+    /* compares: the FP64 operators */
+    static PM_HDM bool above(double x, double c) { return x > c; }
+    static PM_HDM bool iszero(double x) { return x == 0.0; }
+    static PM_HDM double maxc(double a, double c) { return pm_maxc(a, c); }
+    static PM_HDM double minc(double a, double c) { return pm_min(c, a); }
+    static PM_HDM double max_mag(double a, double b) { return pm_max(a, b); }
 };
 #if defined(__CUDA_ARCH__)
 /* device fast paths with a deferred validity flag (pmath.h) */
@@ -316,7 +323,18 @@ struct OpsFast {
     static __device__ __forceinline__ double exp_(double x, unsigned* bad) { return pm_expx_fast(x, bad); }
     static __device__ __forceinline__ double pow_(double x, double y, unsigned* bad) { return pm_pow_fast(x, y, bad); }
     static __device__ __forceinline__ double log_(double x, unsigned* bad) { return pm_log_fast(x, bad); }
+    /* log of an operand that is positive and finite whenever the flag is clear: no special-case selects */
+    static __device__ __forceinline__ double log_pos(double x, unsigned* bad) { return pm_log_core_fast(x, bad); }
     static __device__ __forceinline__ double log10_(double x, unsigned* bad) { return pm_log10_fast(x, bad); }
+    /* compares off the FP64 pipe (pmath.h), each exact for every operand the fast path lets through unflagged:
+       above(x, c) is the test of a clamp x > c ? c : x with c's low word zero, where x == c gives c either way, and
+       x is never NaN unflagged; maxc / minc take an operand that is NaN only if the flag is raised; max_mag two
+       magnitudes */
+    static __device__ __forceinline__ bool above(double x, double c) { return pm_ge_hw(x, c); }
+    static __device__ __forceinline__ bool iszero(double x) { return pm_iszero(x); }
+    static __device__ __forceinline__ double maxc(double a, double c) { return pm_maxc_i(a, c); }
+    static __device__ __forceinline__ double minc(double a, double c) { return pm_minc_i(a, c); }
+    static __device__ __forceinline__ double max_mag(double a, double b) { return pm_max_mag(a, b); }
 };
 #endif
 
@@ -377,13 +395,13 @@ PM_HD void rhs3(const picles_params_t& P, const Hoist& H, double lne, double cx,
     double c_gp = NC ? O::div_pre_nc(O::absnn(cbar), r_g, H.y_rg) : O::div_pre(fabs(cbar), r_g, H.y_rg, bad);
     /* g/(4m) and g/(2m) with the power of two moved into the dividend: the same real quotient,
        hence the same rounded one (neither can leave the normal range), one multiplication less each */
-    double kp = NC ? O::div_nc(9.81 / 4.0, pm_maxc(c_gp * c_gp, 1e-2)) : O::div(9.81 / 4.0, pm_maxc(c_gp * c_gp, 1e-2), bad);
-    double wp = NC ? O::div_nc(9.81 / 2.0, pm_maxc(O::absnn(c_gp), 0.1)) : O::div(9.81 / 2.0, pm_maxc(fabs(c_gp), 0.1), bad);
+    double kp = NC ? O::div_nc(9.81 / 4.0, O::maxc(c_gp * c_gp, 1e-2)) : O::div(9.81 / 4.0, O::maxc(c_gp * c_gp, 1e-2), bad);
+    double wp = NC ? O::div_nc(9.81 / 2.0, O::maxc(O::absnn(c_gp), 0.1)) : O::div(9.81 / 2.0, O::maxc(fabs(c_gp), 0.1), bad);
     double gx = O::divz_pre(cx, r_g, H.y_rg, bad), gy = O::divz_pre(cy, r_g, H.y_rg, bad);
     double a1 = O::div(us, 2.0 * c_gp, bad); /* α_func(us, c_gp) */
-    double alpha = (a1 > 500.0) ? 500.0 : a1;
+    double alpha = O::above(a1, 500.0) ? 500.0 : a1;
     double sg = O::sqrt_(gx * gx + gy * gy, bad);
-    double msg = pm_maxc(sg, 1e-4);
+    double msg = O::maxc(sg, 1e-4);
     double alpha_p = O::div(u * gx + v * gy, 2.0 * (msg * msg), bad);
     /* the fast tanh and sech do not test for NaN: alpha_p is NaN only if its division raised the flag, and with a
        finite p (STD) neither argument can be NaN otherwise */
@@ -410,9 +428,9 @@ PM_HD void rhs3(const picles_params_t& P, const Hoist& H, double lne, double cx,
     double Sdir;
     {
         double a2r = O::div(us, 2.0 * sg, bad); /* α_func(us, sg) */
-        double a2 = (a2r > 500.0) ? 500.0 : a2r;
+        double a2 = O::above(a2r, 500.0) ? 500.0 : a2r;
         double prod = us * sg;
-        bool zero = (prod == 0.0);
+        bool zero = O::iszero(prod);
         double den = zero ? 1.0 : prod * prod;
         double s2 = O::div(2.0, den, bad) *
                     (u * v * (2.0 * (gy * gy) - sg * sg) - gx * gy * (2.0 * (v * v) - us * us));
@@ -635,17 +653,20 @@ PM_HD void step_control(const picles_params_t& P, const Tableau& T, double dt, d
                         double xe, double ye, double u0, double u1, double u2, double u3, double u4, double n0,
                         double n1, double n2, double n3, double n4, double lq, StepCtl& sc, unsigned* bad) {
     const double qmin = 0.2, qmax = 10.0, gamma = 0.9;
-    double r0 = O::divz(dt * e0, fma(pm_max(fabs(u0), fabs(n0)), P.reltol, P.abstol), bad);
-    double r1 = O::divz(dt * e1, fma(pm_max(fabs(u1), fabs(n1)), P.reltol, P.abstol), bad);
-    double r2 = O::divz(dt * e2, fma(pm_max(fabs(u2), fabs(n2)), P.reltol, P.abstol), bad);
-    double r3 = O::divz(dt * xe, fma(pm_max(fabs(u3), fabs(n3)), P.reltol, P.abstol), bad);
-    double r4 = O::divz(dt * ye, fma(pm_max(fabs(u4), fabs(n4)), P.reltol, P.abstol), bad);
+    double r0 = O::divz(dt * e0, fma(O::max_mag(fabs(u0), fabs(n0)), P.reltol, P.abstol), bad);
+    double r1 = O::divz(dt * e1, fma(O::max_mag(fabs(u1), fabs(n1)), P.reltol, P.abstol), bad);
+    double r2 = O::divz(dt * e2, fma(O::max_mag(fabs(u2), fabs(n2)), P.reltol, P.abstol), bad);
+    double r3 = O::divz(dt * xe, fma(O::max_mag(fabs(u3), fabs(n3)), P.reltol, P.abstol), bad);
+    double r4 = O::divz(dt * ye, fma(O::max_mag(fabs(u4), fabs(n4)), P.reltol, P.abstol), bad);
     double EEst = rms5<O>(r0, r1, r2, r3, r4, bad);
-    bool zero = (EEst == 0.0);
-    double lE = O::log_(zero ? 1.0 : EEst, bad);
+    bool zero = O::iszero(EEst);
+    /* EEst = sqrtz(...): with the flag clear it is +0 (replaced by 1) or a positive normal number, so the fast log
+       needs none of its special cases; the exponent below is flagged outside [-700, 700] by the fast exp, whose
+       in-range value is pm_exp's (pmath.h) */
+    double lE = O::log_pos(zero ? 1.0 : EEst, bad);
     double t1 = T.beta1 * lE;
-    double q = pm_exp(t1 - T.beta2 * lq);
-    q = pm_max(1.0 / qmax, pm_min(1.0 / qmin, O::div(q, gamma, bad)));
+    double q = O::exp_(t1 - T.beta2 * lq, bad);
+    q = O::maxc(O::minc(O::div(q, gamma, bad), 1.0 / qmin), 1.0 / qmax);
     sc.EEst = EEst;
     sc.q = zero ? 1.0 / qmax : q;
     sc.t1 = t1;
@@ -923,7 +944,9 @@ PM_HD bool integrate(const picles_params_t& P, const double wu0, const double wv
             step_control_cold(P, T, dt, e0, e1, e2, xe, ye, u0, u1, u2, u3, u4, n0, n1, n2, n3, n4, lq, sc);
 #endif
             double EEst = sc.EEst;
-            const bool accept = (EEst <= 1.0) || (P.force_dtmin && fabs(dt) <= K.ld(KS_DTMIN));
+            /* EEst is a root of a sum of squares: +0 or above, or NaN.  For such operands (and the magnitude |dt|
+               against a positive bound) the compares below are integer compares of the bit patterns (pmath.h) */
+            const bool accept = pm_le_u(EEst, 1.0) || (P.force_dtmin && pm_le_u(fabs(dt), K.ld(KS_DTMIN)));
             /* the step size the controller proposes (and, accepted, the new time) first: the
                AutoSwitch test below needs it while the state of the attempt is still intact */
             double dt_next, t_next = t, dtmin_next = 0.0;
@@ -932,13 +955,13 @@ PM_HD bool integrate(const picles_params_t& P, const double wu0, const double wv
                 double dtnew = dt / sc.q;
                 double ttmp = t + dt;
                 const double tstop = K.ld(KS_TSTOP);
-                t_next = (fabs(ttmp - tstop) < 100.0 * pm_eps(tstop)) ? tstop : ttmp;
+                t_next = pm_lt_u(fabs(ttmp - tstop), 100.0 * pm_eps(tstop)) ? tstop : ttmp; /* bound > 0: tstop finite */
                 double dtp = pm_min(P.dtmax, dtnew);
                 dtmin_next = pm_max(pm_eps(t_next), P.dtmin);
                 dt_next = pm_max(dtp, dtmin_next);
             } else {
                 /* step_reject_controller!: dt /= min(1/qmin, q11/gamma), q11 = EEst^beta1 */
-                double q11 = (EEst == 0.0) ? 1.0 : pm_exp(sc.t1);
+                double q11 = pm_iszero(EEst) ? 1.0 : pm_exp(sc.t1);
 #if defined(__CUDA_ARCH__)
                 /* the specialised copies (TSIT5 != 0) are launched only with the switch off (ph_advance_variant): their
                    code is what it was before the switch existed */
@@ -954,7 +977,7 @@ PM_HD bool integrate(const picles_params_t& P, const double wu0, const double wv
                 is_stiff = stiffness_test(num, den, dt_next);
             }
             if (accept) {
-                bool big = (EEst > PH_QOLDINIT) || (EEst != EEst);
+                bool big = !pm_le_u(EEst, PH_QOLDINIT); /* EEst > qoldinit or NaN */
                 K.st(KS_QOLD, big ? EEst : PH_QOLDINIT); /* max(EEst, qoldinit) */
                 K.st(KS_LQ, big ? sc.lE : LQ0);
                 t = t_next;

@@ -5,8 +5,8 @@
  * No include guard on purpose.  Straight-line code only (selects, no early returns).
  */
 
-/* log(x), fdlibm/musl kernel.  x <= 0, inf, NaN handled by the trailing selects. */
-PM_FN double PMV(pm_log)(double x PM_BADP) {
+/* log(x) for x positive and finite (normal or subnormal), fdlibm/musl kernel */
+PM_FN double PMV(pm_log_core)(double x PM_BADP) {
     uint64_t ub = (uint64_t)pm_d2i(x);
     int sub = ((ub >> 52) == 0); /* +0 or positive subnormal: scale up by 2^54 */
     double xs = sub ? x * 18014398509481984.0 : x;
@@ -29,7 +29,11 @@ PM_FN double PMV(pm_log)(double x PM_BADP) {
     double t2 = z * (PMK.Lg[1] + w * (PMK.Lg[3] + w * (PMK.Lg[5] + w * PMK.Lg[7])));
     double R = t2 + t1;
     double dk = (double)k;
-    double res = s * (hfsq + R) + dk * PMK.LN2_LO - hfsq + f + dk * PMK.LN2_HI;
+    return s * (hfsq + R) + dk * PMK.LN2_LO - hfsq + f + dk * PMK.LN2_HI;
+}
+/* log(x): x <= 0, inf, NaN handled by the trailing selects */
+PM_FN double PMV(pm_log)(double x PM_BADP) {
+    double res = PMV(pm_log_core)(x PM_BADA);
     res = pm_isinf(x) ? x : res;
     res = (x == 0.0) ? -pm_inf() : res;
     res = (x < 0.0) ? pm_nan() : res;
@@ -54,7 +58,13 @@ PM_FN double PMV(pm_pow)(double x, double y PM_BADP) {
 /* tanh(x) = em1/(em1+2), em1 = expm1(2|x|) */
 PM_FN double PMV(pm_tanh)(double x PM_BADP) {
     double ax = fabs(x);
+    /* fast instantiation: the clamps below as high-word compares (pm_ge_hw).  At ax == 25 and ax == 22 both sides of
+       each select give the same value (2*25; tanh(22) rounds to 1), so `>=` is `>` here */
+#ifdef PM_FAST_RANGE
+    double y = pm_ge_hw(ax, 25.0) ? 50.0 : 2.0 * ax;
+#else
     double y = (ax > 25.0) ? 50.0 : 2.0 * ax;
+#endif
 #ifndef PM_FAST_RANGE
     y = (x != x) ? 0.0 : y;
 #endif
@@ -68,7 +78,11 @@ PM_FN double PMV(pm_tanh)(double x PM_BADP) {
     double th = sj * s, tl = sl * s;
     double em1 = fma(th, em, (th - 1.0) + tl);
     double t = PM_DIVZ(em1, em1 + 2.0);
+#ifdef PM_FAST_RANGE
+    t = pm_ge_hw(ax, 22.0) ? 1.0 : t;
+#else
     t = (ax > 22.0) ? 1.0 : t;
+#endif
     t = copysign(t, x); /* t >= 0: one bit operation instead of compare, negate and select */
 #ifdef PM_FAST_RANGE
     return t;
@@ -81,7 +95,11 @@ PM_FN double PMV(pm_tanh)(double x PM_BADP) {
    1 - 1.25*sech^2, where anything below 1e-9 vanishes */
 PM_FN double PMV(pm_sech)(double x PM_BADP) {
     double ax = fabs(x);
+#ifdef PM_FAST_RANGE
+    ax = pm_ge_hw(ax, 350.0) ? 350.0 : ax; /* the same clamp: ties give 350 either way */
+#else
     ax = (ax > 350.0) ? 350.0 : ax;
+#endif
 #ifndef PM_FAST_RANGE
     ax = (x != x) ? 0.0 : ax; /* fast instantiation: NaN is the caller's to flag, as in pm_tanh */
 #endif
@@ -103,7 +121,7 @@ PM_FN double PMV(pm_sech)(double x PM_BADP) {
 /* exp(x): the fast instantiation flags everything outside [-700, 700] (and NaN) */
 PM_FN double PMV(pm_expx)(double x PM_BADP) {
 #ifdef PM_FAST_RANGE
-    *pm_bad |= (fabs(x) <= 700.0) ? 0u : 1u;
+    *pm_bad |= pm_absge_hw(x, 700.0) ? 1u : 0u; /* also flags |x| == 700, which the IEEE instantiation gives the same bits */
     return pm_exp_core_inrange(x);
 #else
     return pm_exp(x);
