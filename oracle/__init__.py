@@ -7,6 +7,7 @@ cpu_baseline / --impl reference legs; never by the product package.  PARITY UNPI
 from __future__ import annotations
 
 import ctypes as C
+import fcntl
 import os
 import subprocess
 
@@ -26,13 +27,23 @@ _VARIANTS = {
 _libs: dict = {}
 
 
-def build(force: bool = False) -> None:
-    """Compile the oracle variants with the committed Makefile."""
-    if force:
-        subprocess.run(["make", "-C", HERE, "clean"], check=True, capture_output=True)
-    r = subprocess.run(["make", "-C", HERE], capture_output=True, text=True)
+def make(*targets: str) -> None:
+    """Run the committed Makefile (every variant when no target is named) under a lock on the build directory, so that
+    processes starting at the same time build each library once and none loads one being written."""
+    os.makedirs(BUILD, exist_ok=True)
+    fd = os.open(os.path.join(BUILD, ".lock"), os.O_RDONLY | os.O_CREAT, 0o644)
+    try:
+        fcntl.flock(fd, fcntl.LOCK_EX)
+        r = subprocess.run(["make", "-s", "-C", HERE, *targets], capture_output=True, text=True)
+    finally:
+        os.close(fd)
     if r.returncode != 0:
         raise RuntimeError("oracle build failed:\n" + r.stdout + r.stderr)
+
+
+def build(force: bool = False) -> None:
+    """Compile the oracle variants with the committed Makefile; `force` rebuilds every one."""
+    make("-B" if force else "all")
 
 
 def _dp(a):
@@ -42,13 +53,8 @@ def _dp(a):
 def load(variant: str = "default"):
     if variant in _libs:
         return _libs[variant]
-    path = os.path.join(BUILD, _VARIANTS[variant])
-    csrc = os.path.join(os.path.dirname(HERE), "picles_b200", "csrc")
-    deps = [os.path.join(HERE, "picles_oracle.c"), os.path.join(os.path.dirname(HERE), "include", "picles_b200.h")]
-    deps += [os.path.join(csrc, h) for h in ("pmath.h", "pmath_body.h", "pmath_trig.h", "pmath_dual.h")]
-    if not os.path.exists(path) or any(os.path.getmtime(path) < os.path.getmtime(d) for d in deps):
-        build()
-    lib = C.CDLL(path)
+    make("_build/" + _VARIANTS[variant])
+    lib = C.CDLL(os.path.join(BUILD, _VARIANTS[variant]))
     vp, d, i64, i32 = C.c_void_p, C.c_double, C.c_int64, C.c_int
     lib.oracle_create.restype = vp
     lib.oracle_create.argtypes = [i32, i32, i32, i32, vp, vp, vp, vp, C.POINTER(PiclesParams)]

@@ -3,14 +3,12 @@ from __future__ import annotations
 
 import ctypes as C
 import os
-import subprocess
 
 import numpy as np
 
+from oracle import BUILD, make
 from picles_b200._abi import PiclesCounters, PiclesParams
 
-HERE = os.path.dirname(os.path.abspath(__file__))
-SO = os.path.join(HERE, "_build", "libpicles_oracle_1d.so")
 _lib = None
 WIND_FN = C.CFUNCTYPE(C.c_double, C.c_double, C.c_double)
 
@@ -18,10 +16,8 @@ WIND_FN = C.CFUNCTYPE(C.c_double, C.c_double, C.c_double)
 def lib():
     global _lib
     if _lib is None:
-        r = subprocess.run(["make", "-s", "-C", HERE, "_build/libpicles_oracle_1d.so"], capture_output=True, text=True)
-        if r.returncode != 0:
-            raise RuntimeError("oracle 1-D build failed:\n" + r.stdout + r.stderr)
-        L = C.CDLL(SO)
+        make("_build/libpicles_oracle_1d.so")
+        L = C.CDLL(os.path.join(BUILD, "libpicles_oracle_1d.so"))
         vp, d = C.c_void_p, C.c_double
         L.oracle1d_create.restype = vp
         L.oracle1d_create.argtypes = [C.c_int, d, d, vp, C.POINTER(PiclesParams)]

@@ -5,10 +5,10 @@ from __future__ import annotations
 import ctypes as C
 import math
 import os
-import subprocess
 
 import numpy as np
 
+import host_build
 import oracle
 from picles_b200 import FetchRelations as FR
 from picles_b200._abi import (BND_NONPERIODIC, BND_PERIODIC, BND_TRIPOLAR_NORTH, PiclesCounters,  # noqa: F401
@@ -18,8 +18,6 @@ from picles_b200.params import make_params
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-SHIM_SRC = os.path.join(HERE, "host_shim.cpp")
-SHIM_SO = os.path.join(HERE, "_build", "libhost_shim.so")
 
 
 def default_params(DT=600.0, solver="Tsit5", dt=1e-3, dtmin=1e-4, force_dtmin=True, periodic_boundary=False,
@@ -77,30 +75,13 @@ def make_oracle(grid, P, variant="default", threads=1):
 
 # ---- host build of the device physics ------------------------------------------------
 
-def _build_shim():
-    deps = [SHIM_SRC, os.path.join(ROOT, "picles_b200", "csrc", "physics.h"),
-            os.path.join(ROOT, "picles_b200", "csrc", "wind_mesh.h"), os.path.join(ROOT, "picles_b200", "csrc", "stiff.h"),
-            os.path.join(ROOT, "picles_b200", "csrc", "pmath_dual.h"),
-            os.path.join(ROOT, "picles_b200", "csrc", "pmath.h"), os.path.join(ROOT, "include", "picles_b200.h")]
-    if os.path.exists(SHIM_SO) and all(os.path.getmtime(SHIM_SO) >= os.path.getmtime(d) for d in deps):
-        return
-    os.makedirs(os.path.dirname(SHIM_SO), exist_ok=True)
-    gxx = "/usr/bin/g++" if os.path.exists("/usr/bin/g++") else "g++"
-    cmd = [gxx, "-O2", "-std=c++17", "-fPIC", "-ffp-contract=off", "-fno-fast-math", "-mfma", "-shared", "-o",
-           SHIM_SO, SHIM_SRC]
-    r = subprocess.run(cmd, capture_output=True, text=True)
-    if r.returncode != 0:
-        raise RuntimeError("host shim build failed:\n" + r.stderr)
-
-
 _shim = None
 
 
 def shim_lib():
     global _shim
     if _shim is None:
-        _build_shim()
-        lib = C.CDLL(SHIM_SO)
+        lib = host_build.load("host_shim", src=os.path.join(HERE, "host_shim.cpp"))
         vp, d, i32, i64 = C.c_void_p, C.c_double, C.c_int, C.c_int64
         lib.shim_create.restype = vp
         lib.shim_create.argtypes = [i32, i32, i32, i32, i32, i32, vp, vp, vp, vp, C.POINTER(PiclesParams)]
@@ -112,6 +93,8 @@ def shim_lib():
         lib.shim_advance_template.argtypes = [C.POINTER(PiclesParams), i32]
         lib.shim_set_wind_midlevels.argtypes = [vp, i32, vp, vp, i64]
         lib.shim_wind_mesh_sample.argtypes = [i32, i32, i32, vp, vp, vp, vp, vp, i64, vp, vp, d, vp, vp]
+        lib.shim_wind_mesh_sample_members.argtypes = [i32, i32, i32, i32, i32, vp, vp, vp, vp, vp, i64, vp, vp, d, vp,
+                                                      vp]
         lib.shim_seed.argtypes = [vp, vp, vp]
         lib.shim_step.argtypes = [vp, d, d, vp, vp, vp, vp]
         lib.shim_get_state.argtypes = [vp, vp]

@@ -7,12 +7,12 @@ import itertools
 import math
 import os
 import re
-import subprocess
 
 import numpy as np
 import pytest
 
 import advance_cases as AC
+import host_build
 from common import HostShim, PiclesParams, ROOT, compare_models, default_params, make_oracle, shim_lib
 
 KERNELS_CU = os.path.join(ROOT, "picles_b200", "csrc", "picles_kernels.cu")
@@ -40,7 +40,7 @@ def _template_head(src, kernel):
 
 
 @pytest.fixture(scope="module")
-def launch_selection(tmp_path_factory):
+def launch_selection():
     """launch_advance and the templates behind it as they stand in picles_kernels.cu, compiled for the host with
     physics.h (ph_advance_variant) and every kernel launch replaced by a call that records its template arguments
     (default arguments filled in by the compiler from the kernels' own template heads), with the launch counter kept
@@ -92,13 +92,10 @@ extern "C" int select_kernels(const picles_params_t* P, int per_node_M, int memb
     return rec_n;
 }}
 """
-    d = tmp_path_factory.mktemp("launch_selection")
-    cpp, so = d / "sel.cpp", d / "libsel.so"
-    cpp.write_text(code)
-    r = subprocess.run(["g++", "-std=c++17", "-O0", "-shared", "-fPIC", "-I", os.path.join(ROOT, "picles_b200", "csrc"),
-                        "-o", str(so), str(cpp)], capture_output=True, text=True)
-    assert r.returncode == 0, r.stderr
-    lib = C.CDLL(str(so))
+    # -O0: the recorder runs no arithmetic, so optimising it would only slow the build; -I: the text includes
+    # physics.h by name
+    lib = host_build.load("launch_selection", text=code,
+                          flags=["-O0", "-I", os.path.join(ROOT, "picles_b200", "csrc")])
     lib.select_kernels.restype = C.c_int
     lib.select_kernels.argtypes = [C.POINTER(PiclesParams), C.c_int, C.c_int, C.c_void_p, C.c_void_p]
     lib.registered.restype = C.c_int

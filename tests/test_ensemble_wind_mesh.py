@@ -4,38 +4,16 @@ mirrored; the model and engine check their arguments."""
 import ctypes as C
 import os
 import re
-import subprocess
 
 import numpy as np
 import pytest
 
 import oracle
-from common import bits_equal
+from common import ROOT, bits_equal, shim_lib
 
 from picles_b200 import _abi
 
-HERE = os.path.dirname(os.path.abspath(__file__))
-ROOT = os.path.dirname(HERE)
-SRC = os.path.join(HERE, "wind_members_shim.cpp")
-SO = os.path.join(HERE, "_build", "libwind_members_shim.so")
 CHUNK = 8  # WM_MEMBER_CHUNK of picles_kernels.cu
-
-
-def shim():
-    deps = [SRC] + [os.path.join(ROOT, "picles_b200", "csrc", h) for h in ("wind_mesh.h", "pmath.h")]
-    if not (os.path.exists(SO) and all(os.path.getmtime(SO) >= os.path.getmtime(d) for d in deps)):
-        os.makedirs(os.path.dirname(SO), exist_ok=True)
-        gxx = "/usr/bin/g++" if os.path.exists("/usr/bin/g++") else "g++"
-        tmp = SO + ".%d" % os.getpid()
-        r = subprocess.run([gxx, "-O2", "-std=c++17", "-fPIC", "-ffp-contract=off", "-fno-fast-math", "-mfma", "-shared",
-                            "-o", tmp, SRC], capture_output=True, text=True)
-        assert r.returncode == 0, r.stderr
-        os.replace(tmp, SO)
-    lib = C.CDLL(SO)
-    vp, i32 = C.c_void_p, C.c_int
-    lib.shim_wind_mesh_sample_members.argtypes = [i32, i32, i32, i32, i32, vp, vp, vp, vp, vp, C.c_int64, vp, vp,
-                                                  C.c_double, vp, vp]
-    return lib
 
 
 def _p(a):
@@ -48,8 +26,8 @@ def sample_members(xw, yw, tw, U, V, x, y, t, chunk=CHUNK):
     U, V = np.ascontiguousarray(U, np.float64), np.ascontiguousarray(V, np.float64)
     x, y = np.ascontiguousarray(x, np.float64), np.ascontiguousarray(y, np.float64)
     u, v = np.full((E, x.size), np.nan), np.full((E, x.size), np.nan)
-    shim().shim_wind_mesh_sample_members(xw.size, yw.size, tw.size, E, chunk, _p(xw), _p(yw), _p(tw), _p(U), _p(V),
-                                         x.size, _p(x), _p(y), float(t), _p(u), _p(v))
+    shim_lib().shim_wind_mesh_sample_members(xw.size, yw.size, tw.size, E, chunk, _p(xw), _p(yw), _p(tw), _p(U), _p(V),
+                                             x.size, _p(x), _p(y), float(t), _p(u), _p(v))
     return u, v
 
 

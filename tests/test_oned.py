@@ -3,12 +3,12 @@ independently, the merge rule as typed, and the DEVICE header (physics1d.h, host
 import ctypes as C
 import math
 import os
-import subprocess
 
 import mpmath as mp
 import numpy as np
 import pytest
 
+import host_build
 from oracle import oned
 from picles_b200._abi import PiclesCounters, PiclesParams
 from scenarios_1d import SCENARIOS_1D, compare_models_1d, grid_1d, params_1d, run_pair_1d
@@ -23,16 +23,7 @@ class Shim1D:
     @classmethod
     def lib(cls):
         if cls._lib is None:
-            src = os.path.join(ROOT, "tests", "host_shim_1d.cpp")
-            so = os.path.join(ROOT, "tests", "_build", "libhost_shim_1d.so")
-            deps = [src] + [os.path.join(ROOT, "picles_b200", "csrc", f) for f in ("physics1d.h", "pmath.h", "pmath_body.h", "pmath_exptab.h")]
-            if not os.path.exists(so) or any(os.path.getmtime(d) > os.path.getmtime(so) for d in deps):
-                os.makedirs(os.path.dirname(so), exist_ok=True)
-                gxx = "/usr/bin/g++" if os.path.exists("/usr/bin/g++") else "g++"
-                r = subprocess.run([gxx, "-O2", "-std=c++17", "-fPIC", "-ffp-contract=off", "-fno-fast-math", "-mfma", "-shared", "-o", so, src],
-                                   capture_output=True, text=True)
-                assert r.returncode == 0, r.stderr
-            L = C.CDLL(so)
+            L = host_build.load("host_shim_1d", src=os.path.join(ROOT, "tests", "host_shim_1d.cpp"))
             vp, d = C.c_void_p, C.c_double
             L.shim1_create.restype = vp
             L.shim1_create.argtypes = [C.c_int, d, d, vp, C.POINTER(PiclesParams)]

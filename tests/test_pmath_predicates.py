@@ -4,10 +4,11 @@ each replaces: at the edges of its stated premise (+-0, subnormals, +-inf, NaNs 
 constants and their neighbours) and on random operands inside it."""
 import ctypes
 import os
-import subprocess
 
 import numpy as np
 import pytest
+
+import host_build
 
 CSRC = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "picles_b200", "csrc")
 
@@ -35,15 +36,8 @@ OPS = {"ge_hw": 0, "absge_hw": 1, "iszero": 2, "maxc_i": 3, "minc_i": 4, "max_ma
 
 
 @pytest.fixture(scope="module")
-def lib(tmp_path_factory):
-    d = tmp_path_factory.mktemp("pmath_predicates")
-    src, so = d / "pred.c", d / "libpred.so"
-    src.write_text(SRC)
-    cc = "/usr/bin/gcc" if os.path.exists("/usr/bin/gcc") else "gcc"
-    r = subprocess.run([cc, "-O2", "-std=c99", "-fPIC", "-ffp-contract=off", "-mfma", "-shared", "-I", CSRC, "-o", str(so),
-                        str(src), "-lm"], capture_output=True, text=True)
-    assert r.returncode == 0, r.stderr
-    L = ctypes.CDLL(str(so))
+def lib():
+    L = host_build.load("pmath_predicates", text=SRC, lang="c99", flags=["-I", CSRC])  # -I: SRC includes pmath.h by name
     dp = ctypes.POINTER(ctypes.c_double)
     L.ev.argtypes = [ctypes.c_int, dp, dp, ctypes.c_long, dp]
 
